@@ -270,6 +270,8 @@ def run_gpu(args):
     barrier()
     launches = _lib.launch_count() - l0
     ms_total = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:        # before the fused variant below overwrites the same buffers
+        dump_outputs(args.dump_outputs, sets[(args.warmup + args.steps - 1) % NSETS])
 
     # the same outputs (z, KL, bound) from ONE launch (cvb_clifford_ps_rsample_bind: the sample's spectrum is known, so the
     # bind needs two transforms instead of three and z is not re-read) -- reported beside the headline, not as it
@@ -427,6 +429,24 @@ def run_gpu(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_ROWS = 1024    # rows of z and of bind(z, roles) written by --dump-outputs: 2 x 16 MB of the 2 x 64 MB
+
+
+def dump_outputs(out_dir, s):
+    """Write what the last timed step returned as float32 .npy files: z and bind(z, roles) on a fixed, seeded sample of
+    DUMP_ROWS rows (ascending row order), KL and entropy for every row.  The inputs and the device RNG are seeded, so
+    two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.randperm(B_ROWS, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    rows = rows.to(s["z"].device)
+    arrays = {"z": s["z"].index_select(0, rows), "bound": s["out"].index_select(0, rows), "kl": s["kl"],
+              "entropy": s["ent"]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def vae_train_leg(torch, dev, world, rank, local, steps=8, warmup=3, compare_reference_dists=True):
@@ -702,7 +722,14 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true", help="skip the C1/C2/C3-bwd/C4/C5 legs (other_configs)")
     ap.add_argument("--no-vae-step", action="store_true", help="skip the C3 VAE training-step leg (vae_train_step)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's z, bind(z, roles) (seeded sample of rows), KL and "
+                         "entropy to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

@@ -1,6 +1,7 @@
 """CPU-side checks of the drop-in boundary: the shared library loads and exports every symbol that
 include/clifford_b200.h declares (no compute without a GPU), the ctypes table matches the header,
-and the product path refuses CPU tensors instead of falling back."""
+and the product path never computes on the host: the distributions refuse CPU tensors, and the VSA ops stage CPU
+operands to the GPU when one exists and refuse them when none does."""
 import ctypes
 import os
 import re
@@ -41,11 +42,18 @@ def test_ctypes_arity_matches_header():
 
 
 def test_no_cpu_fallback():
+    from clifford_b200 import _lib
     from clifford_b200._lib import CliffordB200Error
     from utils import vsa
     from dists.clifford import CliffordPowerSphericalDistribution, PowerSpherical
-    with pytest.raises(CliffordB200Error):
-        vsa.bind(torch.randn(2, 64), torch.randn(2, 64))
+    a, b = torch.randn(2, 64), torch.randn(2, 64)
+    if torch.cuda.is_available():
+        # the VSA ops stage CPU operands to the GPU (tests/test_gpu_boundary.py): the library's kernel computes them
+        n0 = _lib.launch_count()
+        assert vsa.bind(a, b).device.type == "cpu" and _lib.launch_count() > n0
+    else:
+        with pytest.raises(CliffordB200Error):
+            vsa.bind(a, b)
     with pytest.raises(CliffordB200Error):
         CliffordPowerSphericalDistribution(torch.zeros(2, 16), torch.ones(2, 1)).rsample()
     with pytest.raises(CliffordB200Error):
