@@ -37,6 +37,9 @@ _SIGNATURES = {
     "cvb_clifford_spectrum_adjoint": ([_f, _f, _ll, _i, _f], _i),
     "cvb_ps_entropy_kl": ([_f, _ll, _i, _ll, _i, _db, _i, _db, _f, _f, _f, _f], _i),
     "cvb_clifford_vm_rsample": ([_f, _f, _ll, _i, _ll, _ull, _ull, _f, _ll, _i, _f], _i),
+    "cvb_clifford_vm_rsample_kl": ([_f, _f, _ll, _i, _ll, _ull, _ull, _f, _f, _f, _f, _f, _ll, _i, _f], _i),
+    "cvb_clifford_vm_rsample_backward": ([_f, _f, _f, _ll, _i, _ll, _f, _f, _f, _ll, _i, _f], _i),
+    "cvb_clifford_vm_log_prob": ([_f, _f, _f, _ll, _i, _ll, _f, _f, _f, _f, _ll, _i, _f], _i),
     "cvb_clifford_phases_to_vector": ([_f, _fl, _ull, _ull, _f, _ll, _i, _f], _i),
     "cvb_vsa_bind": ([_f, _f, _f, _ll, _ll, _ll, _i, _i, _f], _i),
     "cvb_vsa_depth_chain_cosine": ([_f, _f, _ll, _i, _i, _f], _i),

@@ -188,10 +188,15 @@ class CliffordTorusDistribution(Distribution):
 
     ``rsample`` draws the von Mises phases on the device (Best & Fisher rejection, the algorithm of
     torch.distributions.VonMises.sample that the reference calls at :262) and maps them through the same Hermitian
-    spectrum -> inverse FFT kernel as the other samplers.  Like the reference's VonMises draw it is NOT reparameterised
-    (no gradient reaches loc / concentration).  The reference's own method never gets that far: its Hermitian-symmetry
+    spectrum -> inverse FFT kernel as the other samplers.  It is reparameterised: under autograd the launch saves the
+    drawn offsets and the backward applies the implicit reparameterisation gradient of every von Mises draw (Figurnov et
+    al. 2018; DESIGN.md section 6), so the reconstruction term reaches loc and concentration.  For one concentration per
+    row the same launch yields the entropy, cached for ``entropy()`` / ``kl_divergence``.  Without a graph it is the
+    plain sampling launch (same draws).  The reference's own method never gets that far: its Hermitian-symmetry
     assert (:274) compares against the wrong flip and raises for generic angles, so no driver uses it
     (scripts/sample_viz.py:55-64 restates the sampler inline); this is the working version of what it computes.
+    ``log_prob`` sums kappa cos(angle(rfft(value)_k) - loc_k) - ln(2 pi I0(kappa)) over circles k >= 1 -- the circles of
+    the entropy and of the uniform prior -- in one kernel with its value / loc / concentration gradients.
     ``entropy`` is one kernel (`cvb_clifford_vm_entropy`: the reference's eps-regularised i0e/i1e expression, evaluated
     from the fp64 log I_v of csrc/special.cuh, with its kappa-derivative).
     """
@@ -203,30 +208,54 @@ class CliffordTorusDistribution(Distribution):
         self._raw_concentration = concentration
         self.loc, self.concentration = broadcast_all(loc, concentration)
         self.orig_dim = loc.shape[-1]
+        self._fused_entropy = None
         super().__init__(batch_shape=loc.shape[:-1], event_shape=torch.Size([2 * self.orig_dim]),
                          validate_args=validate_args)
+
+    def _vm_kappa(self, row_scalar_if_expanded=False):
+        """(rows, 1) for one concentration per row, else (rows, d).  row_scalar_if_expanded: a stride-0 expanded
+        concentration also counts as one per row."""
+        d = self.orig_dim
+        raw = self._raw_concentration
+        if torch.is_tensor(raw) and raw.dim() >= 1 and raw.shape[-1] == 1 and d != 1:
+            return raw.expand(tuple(self.batch_shape) + (1,)).reshape(-1, 1)
+        conc = self.concentration
+        if row_scalar_if_expanded and conc.dim() >= 1 and conc.stride(-1) == 0:
+            return conc[..., :1].reshape(-1, 1)
+        return conc.reshape(-1, d)
 
     def rsample(self, sample_shape=torch.Size()):
         sample_shape = torch.Size(sample_shape)
         d = self.orig_dim
         n = _numel(sample_shape)
-        raw = self._raw_concentration
-        if torch.is_tensor(raw) and raw.dim() >= 1 and raw.shape[-1] == 1 and d != 1:
-            kap = raw.expand(tuple(self.batch_shape) + (1,)).reshape(-1, 1)
+        loc2 = self.loc.reshape(-1, d)
+        kap = self._vm_kappa(row_scalar_if_expanded=True)
+        if torch.is_grad_enabled() and (loc2.requires_grad or kap.requires_grad):
+            z, ent, dent = ops.CliffordVMRsample.apply(loc2, kap, n, True)
+            if ent.numel():                                         # same launch; entropy() / kl_divergence reuse it
+                self._fused_entropy = ops.row_scalar(kap, ent, dent).reshape(self.batch_shape)
         else:
-            kap = self.concentration.reshape(-1, d)
-        z = ops.clifford_vm_rsample(self.loc.reshape(-1, d), kap, n)
+            z = ops.clifford_vm_rsample(loc2, self._vm_kappa(), n)
         return z.reshape(tuple(sample_shape) + tuple(self.batch_shape) + (2 * d,)).to(self.loc.dtype)
 
+    def log_prob(self, value):
+        d = self.orig_dim
+        lead = torch.broadcast_shapes(value.shape[:-1], tuple(self.batch_shape))
+        v2 = value.expand(tuple(lead) + (2 * d,)).reshape(-1, 2 * d)
+        lp = ops.CliffordVMLogProb.apply(v2, self.loc.reshape(-1, d), self._vm_kappa(row_scalar_if_expanded=True))
+        return lp.reshape(lead).to(self.loc.dtype)
+
     def entropy(self):
+        cached = self.__dict__.get("_fused_entropy")
+        if cached is not None:
+            # a value cached without a graph carries none: recompute when the caller now wants d entropy / d kappa
+            kap = self._vm_kappa(row_scalar_if_expanded=True)
+            stale = torch.is_grad_enabled() and kap.requires_grad and cached.grad_fn is None and not cached.requires_grad
+            if not stale:
+                return cached.to(self.loc.dtype)
         # one kernel: sum over circles k >= 1 of ln 2 pi + ln(i0e + eps) + kappa - kappa (i1e + eps) / (i0e + eps)
         d = self.orig_dim
-        raw = self._raw_concentration
-        if torch.is_tensor(raw) and raw.dim() >= 1 and raw.shape[-1] == 1 and d != 1:
-            kap = raw.expand(tuple(self.batch_shape) + (1,)).reshape(-1, 1)
-        else:
-            kap = self.concentration.reshape(-1, d)
-        ent = ops.VMTorusEntropy.apply(kap, d)
+        ent = ops.VMTorusEntropy.apply(self._vm_kappa(), d)
         return ent.reshape(self.batch_shape).to(self.loc.dtype)
 
 

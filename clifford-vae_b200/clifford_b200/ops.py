@@ -247,48 +247,123 @@ class PSEntropy(torch.autograd.Function):
         return dk.reshape(ctx.kshape), None, None, None
 
 
+def _torus_log_prob_forward(ctx, entry, value, loc, kappa):
+    """The launch of a Clifford-torus log_prob (`entry`: the power-spherical or the von Mises family) with the derivative
+    outputs autograd will need, saved on ctx for _torus_log_prob_backward."""
+    lib, dev = _prep(value, loc, kappa)
+    B, d = loc.shape
+    rows = value.shape[0]
+    val_c, loc_c = _f32c(value), _f32c(loc)
+    kap_c, krs, kes = _kappa_layout(kappa, d)
+    lp = torch.empty(rows, device=dev, dtype=torch.float32)
+    need = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+    dl = torch.empty(rows, d, device=dev, dtype=torch.float32) if need else None
+    dk = torch.empty((rows,) if kes == 0 else (rows, d), device=dev, dtype=torch.float32) if need else None
+    dF = torch.empty(rows, d, 2, device=dev, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+    _launch(entry, dev, ptr(val_c), ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(lp), ptr(dl), ptr(dk), ptr(dF), rows, d,
+            skip=rows == 0 or d == 0)
+    ctx.save_for_backward(dl, dk, dF)
+    ctx.meta = (B, d, rows, kes, tuple(kappa.shape))
+    return lp
+
+
+def _torus_log_prob_backward(ctx, grad):
+    dl, dk, dF = ctx.saved_tensors
+    B, d, rows, kes, kshape = ctx.meta
+    S = rows // B if B else 0
+    g = grad.reshape(rows)
+    dval = dloc = dkap = None
+    if dF is not None:
+        h = (g[:, None, None] * dF).contiguous()
+        dval = torch.empty(rows, 2 * d, device=g.device, dtype=torch.float32)
+        _launch("cvb_clifford_spectrum_adjoint", g.device, ptr(h), ptr(dval), rows, d, skip=rows == 0 or d == 0)
+    if dl is not None:
+        dloc = (g[:, None] * dl).view(S, B, d).sum(0)
+        dkap = ((g * dk).view(S, B).sum(0) if kes == 0 else (g[:, None] * dk).view(S, B, d).sum(0)).reshape(kshape)
+    return dval, dloc, dkap
+
+
 class CliffordPSLogProb(torch.autograd.Function):
     """log_prob (rows,) of value (rows, 2d) under (loc (B,d), kappa (B,1)|(B,d)); rows = S*B.
     Differentiable in loc, kappa and value (the value gradient goes through the adjoint of the truncated real FFT)."""
 
     @staticmethod
     def forward(ctx, value, loc, kappa):
-        lib, dev = _prep(value, loc, kappa)
-        B, d = loc.shape
-        rows = value.shape[0]
-        val_c, loc_c = _f32c(value), _f32c(loc)
-        kap_c, krs, kes = _kappa_layout(kappa, d)
-        lp = torch.empty(rows, device=dev, dtype=torch.float32)
-        need = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-        dl = torch.empty(rows, d, device=dev, dtype=torch.float32) if need else None
-        dk = torch.empty((rows,) if kes == 0 else (rows, d), device=dev, dtype=torch.float32) if need else None
-        dF = torch.empty(rows, d, 2, device=dev, dtype=torch.float32) if ctx.needs_input_grad[0] else None
-        _launch("cvb_clifford_ps_log_prob", dev, ptr(val_c), ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(lp), ptr(dl),
-                ptr(dk), ptr(dF), rows, d, skip=rows == 0 or d == 0)
-        ctx.save_for_backward(dl, dk, dF)
-        ctx.meta = (B, d, rows, kes, tuple(kappa.shape))
-        return lp
+        return _torus_log_prob_forward(ctx, "cvb_clifford_ps_log_prob", value, loc, kappa)
 
     @staticmethod
     def backward(ctx, grad):
-        dl, dk, dF = ctx.saved_tensors
-        B, d, rows, kes, kshape = ctx.meta
-        S = rows // B
-        g = grad.reshape(rows)
-        dval = dloc = dkap = None
-        if dF is not None:
-            h = (g[:, None, None] * dF).contiguous()
-            dval = torch.empty(rows, 2 * d, device=g.device, dtype=torch.float32)
-            _launch("cvb_clifford_spectrum_adjoint", g.device, ptr(h), ptr(dval), rows, d, skip=rows == 0 or d == 0)
-        if dl is not None:
-            dloc = (g[:, None] * dl).view(S, B, d).sum(0)
-            dkap = ((g * dk).view(S, B).sum(0) if kes == 0 else (g[:, None] * dk).view(S, B, d).sum(0)).reshape(kshape)
-        return dval, dloc, dkap
+        return _torus_log_prob_backward(ctx, grad)
+
+
+class CliffordVMLogProb(torch.autograd.Function):
+    """von Mises torus log_prob (rows,) of value (rows, 2d) under (loc (B,d), kappa (B,1)|(B,d)); rows = S*B: the sum over
+    circles k >= 1 of kappa cos(angle(rfft(value)_k) - loc_k) - ln(2 pi I0(kappa)).  Differentiable in value, loc, kappa."""
+
+    @staticmethod
+    def forward(ctx, value, loc, kappa):
+        return _torus_log_prob_forward(ctx, "cvb_clifford_vm_log_prob", value, loc, kappa)
+
+    @staticmethod
+    def backward(ctx, grad):
+        return _torus_log_prob_backward(ctx, grad)
+
+
+class CliffordVMRsample(torch.autograd.Function):
+    """z, entropy = f(loc (B,d), kappa (B,1)|(B,d)) for the von Mises torus; rows = n_samples * B.  The same draws as
+    clifford_vm_rsample for the same generator state; the launch also saves the drawn offsets phi for the backward
+    (the implicit reparameterisation gradient of every von Mises draw, cvb_clifford_vm_rsample_backward).
+    Returns (z (rows, 2d), entropy (B,), d entropy / d kappa (B,)); the last two are plain values (empty when kappa is per
+    element, n_samples > 1 or want_entropy is false) that the distribution re-attaches to kappa with row_scalar()."""
+
+    @staticmethod
+    def forward(ctx, loc, kappa, n_samples, want_entropy):
+        lib, dev = _prep(loc, kappa)
+        B, d = loc.shape
+        rows = B * n_samples
+        loc_c = _f32c(loc)
+        kap_c, krs, kes = _kappa_layout(kappa, d)
+        z = torch.empty(rows, 2 * d, device=dev, dtype=torch.float32)
+        need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        phi = torch.empty(rows, d, device=dev, dtype=torch.float32) if need_grad else None
+        fused_ent = bool(want_entropy) and kes == 0 and n_samples == 1
+        ent = torch.empty(B, device=dev, dtype=torch.float32) if fused_ent else None
+        dent = torch.empty(B, device=dev, dtype=torch.float32) if fused_ent else None
+        seed, off = _lib.next_rng(dev)
+        _launch("cvb_clifford_vm_rsample_kl", dev, ptr(loc_c), ptr(kap_c), krs, kes, B, seed, off, ptr(z), ptr(phi),
+                ptr(ent), None, ptr(dent), rows, d, skip=rows == 0 or d == 0)
+        ctx.save_for_backward(loc_c, kap_c, phi)
+        ctx.meta = (B, d, rows, n_samples, krs, kes, tuple(kappa.shape))
+        if ent is None:
+            ent, dent = z.new_empty(0), z.new_empty(0)
+        ctx.mark_non_differentiable(ent, dent)      # re-attached to kappa by row_scalar(): its own autograd node
+        return z, ent, dent
+
+    @staticmethod
+    def backward(ctx, grad_z, grad_ent, grad_dent):
+        loc_c, kap_c, phi = ctx.saved_tensors
+        B, d, rows, n_samples, krs, kes, kshape = ctx.meta
+        dloc = dkap = None
+        if grad_z is not None and phi is not None:
+            gz = _f32c(grad_z)
+            dloc_rows = torch.empty(rows, d, device=gz.device, dtype=torch.float32)
+            dk_rows = torch.empty((rows,) if kes == 0 else (rows, d), device=gz.device, dtype=torch.float32)
+            _launch("cvb_clifford_vm_rsample_backward", gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(phi),
+                    ptr(dloc_rows), ptr(dk_rows), rows, d, skip=rows == 0 or d == 0)
+            if n_samples > 1:
+                dloc_rows = dloc_rows.view(n_samples, B, d).sum(0)
+                dk_rows = dk_rows.view(n_samples, B, -1).sum(0) if kes else dk_rows.view(n_samples, B).sum(0)
+            dloc = dloc_rows
+            dkap = dk_rows.reshape(kshape)
+        if dloc is None and ctx.needs_input_grad[0]:
+            dloc = torch.zeros_like(loc_c)
+        return dloc, dkap, None, None
 
 
 def clifford_vm_rsample(loc, kappa, n_samples=1):
     """z (n_samples * B, 2d) of the von Mises torus distribution (dists/clifford.py:261-275): phases loc + VonMises(0, kappa)
-    drawn on the device, then the Hermitian-spectrum inverse FFT.  loc (B, d), kappa (B, 1) | (B, d).  No autograd."""
+    drawn on the device, then the Hermitian-spectrum inverse FFT.  loc (B, d), kappa (B, 1) | (B, d).  Forward only (the
+    sampling path without a graph); CliffordVMRsample draws the same z with a backward."""
     lib, dev = _prep(loc, kappa)
     B, d = loc.shape
     rows = B * n_samples

@@ -11,17 +11,17 @@ namespace {
 
 constexpr size_t kGenericSmemLimit = 200 * 1024;
 
-template <int LOG2N, bool ROWK, bool FAST = false>
+template <int LOG2N, bool ROWK, bool FAST = false, bool VM = false>
 int launch_bwd_fast(const CliffordBwdParams& p, cudaStream_t st) {
-  if constexpr (ROWK && !FAST) {
+  if constexpr (ROWK && !FAST && !VM) {
     if (p.tp_signed && p.staged) return launch_bwd_fast<LOG2N, ROWK, true>(p, st);   // the training path
   }
   using Pl = FftPlan<LOG2N>;
   const cplx* tw = device_twiddles();
   const float2* icdf = device_icdf_table();
   if (!tw || !icdf) return kCudaError;
-  const size_t smem = clifford_bwd_smem_bytes<LOG2N, ROWK, FAST>();
-  auto kern = clifford_bwd_kernel<LOG2N, ROWK, FAST>;
+  const size_t smem = clifford_bwd_smem_bytes<LOG2N, ROWK, FAST, VM>();
+  auto kern = clifford_bwd_kernel<LOG2N, ROWK, FAST, VM>;
   int grid = 0;
   const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
   if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
@@ -32,7 +32,7 @@ int launch_bwd_fast(const CliffordBwdParams& p, cudaStream_t st) {
   return check_launch("clifford_bwd_kernel");
 }
 
-template <bool ROWK>
+template <bool ROWK, bool VM = false>
 int dispatch_bwd(const CliffordBwdParams& p_in, cudaStream_t st) {
   CliffordBwdParams p = p_in;
   p.staged = aligned(p.loc, 16) && (!p.tp_signed || aligned(p.tp_signed, 16)) && (!p.tprime || aligned(p.tprime, 16)) &&
@@ -40,7 +40,7 @@ int dispatch_bwd(const CliffordBwdParams& p_in, cudaStream_t st) {
   const bool fast = is_pow2(p.d) && p.d >= 16 && p.d <= 8192 && aligned(p.grad_z, 8);
   if (fast) {
     switch (ilog2(p.d)) {
-#define CVB_CASE(L) case L: return launch_bwd_fast<L, ROWK>(p, st);
+#define CVB_CASE(L) case L: return launch_bwd_fast<L, ROWK, false, VM>(p, st);
       CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
       CVB_CASE(13)
 #undef CVB_CASE
@@ -50,7 +50,7 @@ int dispatch_bwd(const CliffordBwdParams& p_in, cudaStream_t st) {
   if (2 * p.d <= kSmallMaxN && !no_small) {
     const int rt = small_rows_per_tile(p.rows, sm_count(), [&](int r) { return clifford_bwd_small_smem(p.d, r); });
     const size_t smem_s = clifford_bwd_small_smem(p.d, rt);
-    auto kern_s = clifford_bwd_small_kernel<ROWK>;
+    auto kern_s = clifford_bwd_small_kernel<ROWK, VM>;
     int grid_s = 0;
     if (int rc = persistent_grid(kern_s, kSmallThreads, smem_s, (p.rows + rt - 1) / rt, &grid_s)) return rc;
     kern_s<<<grid_s, kSmallThreads, smem_s, st>>>(p, rt);
@@ -59,7 +59,7 @@ int dispatch_bwd(const CliffordBwdParams& p_in, cudaStream_t st) {
   const int n = 2 * p.d;
   const size_t smem = sizeof(cplx) * n + sizeof(float) * (n + 32);
   CVB_REQUIRE(smem <= kGenericSmemLimit, kUnsupported, "clifford backward: d=%d too large for the direct-DFT path", p.d);
-  auto kern = clifford_bwd_generic_kernel<ROWK>;
+  auto kern = clifford_bwd_generic_kernel<ROWK, VM>;
   int grid = 0;
   if (int rc = persistent_grid(kern, kGenericThreads, smem, p.rows, &grid)) return rc;
   kern<<<grid, kGenericThreads, smem, st>>>(p);
@@ -116,6 +116,20 @@ int cvb_ps_entropy_kl(const float* kappa, long long kappa_row_stride, int kappa_
   if (blocks > cap) blocks = cap;
   ps_entropy_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(p);
   return check_launch("ps_entropy_kernel");
+}
+
+// Backward of cvb_clifford_vm_rsample_kl: phi (rows, d) = the offsets that launch saved
+int cvb_clifford_vm_rsample_backward(const float* grad_z, const float* loc, const float* kappa, long long kappa_row_stride,
+                                     int kappa_el_stride, long long loc_rows, const float* phi, float* dloc, float* dkappa,
+                                     long long rows, int d, void* stream) {
+  CVB_REQUIRE(grad_z && loc && kappa && phi && dloc && dkappa, kBadArgument, "cvb_clifford_vm_rsample_backward: null pointer");
+  CVB_REQUIRE(rows > 0 && d >= 1 && loc_rows > 0, kBadArgument, "cvb_clifford_vm_rsample_backward: bad sizes");
+  CliffordBwdParams p{};
+  p.grad_z = grad_z; p.loc = loc; p.kappa = kappa; p.kappa_row_stride = kappa_row_stride;
+  p.kappa_el_stride = kappa_el_stride; p.loc_rows = (int)loc_rows; p.tp_signed = phi; p.dloc = dloc; p.dkappa = dkappa;
+  p.rows = rows; p.d = d;
+  cudaStream_t st = (cudaStream_t)stream;
+  return kappa_el_stride == 0 ? dispatch_bwd<true, true>(p, st) : dispatch_bwd<false, true>(p, st);
 }
 
 // CliffordTorusDistribution.entropy (dists/clifford.py:21-31, :277-278): sum over circles k >= 1 of the von Mises entropy

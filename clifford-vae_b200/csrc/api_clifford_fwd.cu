@@ -196,6 +196,23 @@ int cvb_clifford_vm_rsample(const float* loc, const float* kappa, long long kapp
   return dispatch_fwd<kVonMisesRng, false>(p, (cudaStream_t)stream);
 }
 
+// the same draws (same key, same kernels) with the offsets phi saved for cvb_clifford_vm_rsample_backward and, for one
+// concentration per row, the row entropy / KL to the uniform prior / dH/dkappa of vm_entropy_kernel in the same launch
+int cvb_clifford_vm_rsample_kl(const float* loc, const float* kappa, long long kappa_row_stride, int kappa_el_stride,
+                               long long loc_rows, unsigned long long seed, unsigned long long offset, float* z, float* phi,
+                               float* entropy, float* kl, float* dentropy, long long rows, int d, void* stream) {
+  CVB_REQUIRE(loc && kappa && z, kBadArgument, "cvb_clifford_vm_rsample_kl: null pointer");
+  CVB_REQUIRE(rows > 0 && d >= 1 && loc_rows > 0, kBadArgument, "cvb_clifford_vm_rsample_kl: rows=%lld d=%d loc_rows=%lld", rows, d, loc_rows);
+  CVB_REQUIRE(kappa_el_stride == 0 || (!entropy && !kl && !dentropy), kBadArgument,
+              "cvb_clifford_vm_rsample_kl: fused entropy/kl needs one concentration per row; use cvb_clifford_vm_entropy");
+  CliffordFwdParams p{};
+  p.loc = loc; p.kappa = kappa; p.kappa_row_stride = kappa_row_stride; p.kappa_el_stride = kappa_el_stride;
+  p.loc_rows = (int)loc_rows; p.z = z; p.tp_signed = phi; p.entropy = entropy; p.kl = kl; p.dentropy = dentropy;
+  p.rows = rows; p.d = d; p.n = 2 * d;
+  p.key = make_key(seed, offset, 3);
+  return dispatch_fwd<kVonMisesRng, false>(p, (cudaStream_t)stream);
+}
+
 // fused sample + entropy/KL + bind with a second vector (one concentration per row; power-of-two d in [16, 8192])
 int cvb_clifford_ps_rsample_bind(const float* loc, const float* kappa, long long loc_rows, const float* tprime,
                                  const float* gnoise, unsigned long long seed, unsigned long long offset, const float* b,

@@ -68,7 +68,8 @@ struct CliffordFwdParams {
   const float* phases;     // (rows, d)                               [kPhases]
   float phase_scale;       //                                         [kPhases]; eps for kUnitaryRng
   float* z;                // (rows, n) out
-  float* tp_signed;        // (rows, d) out, optional: copysign(t', s) saved for backward [kPsRng]
+  float* tp_signed;        // (rows, d) out, optional: copysign(t', s) saved for backward [kPsRng]; the von Mises offset
+                           // phi [kVonMisesRng]
   float* entropy;          // (rows) out, optional (row-scalar kappa only)
   float* kl;               // (rows) out, optional (row-scalar kappa only)
   float* dentropy;         // (rows) out, optional: d entropy / d kappa (row-scalar kappa only)
@@ -166,7 +167,8 @@ __device__ __forceinline__ cplx ps_phasor(float tp, float sgn, float loc) {
 
 // One von Mises(0, kappa) draw by Best & Fisher's wrapped-Cauchy rejection, in double like the sampler the reference
 // calls (torch/distributions/von_mises.py:93-190 `_rejection_sample` + `_proposal_r` with its small-kappa Taylor
-// branch); acceptance >= 0.66.  Not reparameterised (VonMises has no rsample): no backward.
+// branch); acceptance >= 0.66.  Its pathwise gradient is the implicit one of vm_dphi_dkappa below (the draw itself is
+// not a differentiable function of kappa).
 __device__ __forceinline__ float von_mises_draw(float kappa_f, const PhiloxKey& key, uint64_t elem) {
   const double kap = (double)kappa_f;
   const double tau = 1.0 + sqrt(1.0 + 4.0 * kap * kap);
@@ -185,6 +187,111 @@ __device__ __forceinline__ float von_mises_draw(float kappa_f, const PhiloxKey& 
     }
   }
   return (float)x;
+}
+
+// Row constants of the von Mises circle law, fp64 -> fp32: b = 1 - A(kappa), A = I1/I0 (kept as 1 - A: it is 1/(2 kappa)
+// for large kappa and every use subtracts from 1), and lnk = ln(2 pi I0(kappa)) - kappa = ln 2 pi + log_ive(0, kappa)
+// (the log-normaliser without its kappa, which the log density cancels against kappa cos: see vm_lp_element).
+// kappa <= 0 (or NaN) is the uniform circle.
+struct VmRowConsts { float b, lnk; };
+__device__ __forceinline__ VmRowConsts vm_row_consts(float kappa_f) {
+  const double k = (double)kappa_f;
+  VmRowConsts c;
+  if (k > 0.0) {
+    const double l0 = log_ive(0.0, k), l1 = log_ive(1.0, k);
+    c.b = (float)(-expm1(l1 - l0));
+    c.lnk = (float)(1.83787706640934548356 + l0);
+  } else {
+    c.b = 1.0f;
+    c.lnk = 1.83787706640934548356f;
+  }
+  return c;
+}
+
+// Implicit reparameterisation gradient of a von Mises(0, kappa) draw phi (Figurnov et al. 2018): phi stays at its CDF
+// level, d phi / d kappa = -d_kappa F / f, which the even symmetry and int_{-pi}^{pi} (cos t - A) e^{kappa cos t} dt = 0
+// reduce to
+//   J(phi) = -int_0^phi (cos t - A) e^{kappa (cos t - cos phi)} dt = +int_phi^pi (cos t - A) e^{kappa (cos t - cos phi)} dt
+// (odd in phi; -sin phi as kappa -> 0).  fp32, 12-point Gauss-Legendre per panel, b = 1 - A from vm_row_consts.  With
+// S = sin(phi/2), C = cos(phi/2), x = kappa (1 - cos phi) = 2 kappa S^2:
+//   x <= 3 (the bulk of every law): the first form on [0, |phi|] in t; the exponent lies in [0, x], the integrand is
+//     smooth, and kappa (cos t - cos phi) = 2 kappa sin((phi+t)/2) sin((phi-t)/2), cos t - A = b - 2 sin^2(t/2) keep
+//     their relative accuracy when kappa is large;
+//   x > 3 (tail draws): the second form, whose integrand has one sign and exponent <= 0 (the first form cancels e^x-sized
+//     halves there).  With s = sin(t/2), s^2 = S^2 + C^2 sin^2 psi it is
+//       int_0^{pi/2} ((cos phi - A) - 2 C^2 sin^2 psi) e^{-2 kappa C^2 sin^2 psi} 2 C sin psi / sqrt(S^2 + C^2 sin^2 psi) dpsi,
+//     integrated on [pi/4, pi/2] in psi (skipped once e^{-kappa C^2} is below fp32 resolution) and on [0, pi/4] in
+//     eta, C sin psi = S sinh eta, which removes the branch point near psi = 0: the integrand becomes
+//     ((cos phi - A) - 2 S^2 sinh^2 eta) e^{-x sinh^2 eta} 2 tan psi, cut where x sinh^2 eta = 40.
+// Against fp64 adaptive quadrature over kappa in [1e-6, 1e4] and phi up to pi: <= 6.2e-7 max(1, |J|) (12 nodes; 8 give
+// 1.5e-5).  Finite for every finite (phi, kappa >= 0): every exponent is <= 3.
+__device__ __forceinline__ float vm_dphi_dkappa(float phi, float kap, float b) {
+  constexpr float kNode[12] = {9.219682877e-03f, 4.794137181e-02f, 1.150486629e-01f, 2.063410229e-01f, 3.160842505e-01f,
+                               4.373832957e-01f, 5.626167043e-01f, 6.839157495e-01f, 7.936589771e-01f, 8.849513371e-01f,
+                               9.520586282e-01f, 9.907803171e-01f};
+  constexpr float kWeight[12] = {2.358766819e-02f, 5.346966300e-02f, 8.003916427e-02f, 1.015837134e-01f, 1.167462683e-01f,
+                                 1.245735229e-01f, 1.245735229e-01f, 1.167462683e-01f, 1.015837134e-01f, 8.003916427e-02f,
+                                 5.346966300e-02f, 2.358766819e-02f};     // Gauss-Legendre on [0, 1]
+  const float a = fabsf(phi);
+  float S, C;
+  sincosf(0.5f * a, &S, &C);
+  const float x = 2.0f * kap * S * S;
+  float J;
+  if (!(x > 3.0f)) {
+    float acc = 0.0f;
+#pragma unroll
+    for (int i = 0; i < 12; ++i) {
+      const float t = a * kNode[i];
+      const float st = sinf(0.5f * t);
+      const float e = 2.0f * kap * sinf(0.5f * (a + t)) * sinf(0.5f * (a - t));
+      acc = fmaf(kWeight[i], fmaf(-2.0f * st, st, b) * expf(e), acc);
+    }
+    J = -a * acc;
+  } else {
+    const float cma = fmaf(-2.0f * S, S, b);                  // cos phi - A  (< 0 here)
+    const float r = S / C;
+    const float e1 = asinhf(fminf(0.70710678f / r, sqrtf(40.0f / x)));
+    float acc = 0.0f;
+#pragma unroll
+    for (int i = 0; i < 12; ++i) {
+      const float sh = sinhf(e1 * kNode[i]);
+      const float sp = r * sh;                                // sin psi <= 1/sqrt 2
+      const float tanp = sp * rsqrtf(fmaf(-sp, sp, 1.0f));
+      acc = fmaf(kWeight[i], fmaf(-2.0f * S * S, sh * sh, cma) * expf(-x * sh * sh) * 2.0f * tanp, acc);
+    }
+    J = e1 * acc;
+    if (kap * C * C < 40.0f) {
+      float acc2 = 0.0f;
+#pragma unroll
+      for (int i = 0; i < 12; ++i) {
+        const float sp = sinf(0.78539816f * (1.0f + kNode[i]));
+        const float c2s2 = C * C * sp * sp;
+        acc2 = fmaf(kWeight[i], fmaf(-2.0f, c2s2, cma) * expf(-2.0f * kap * c2s2) * 2.0f * C * sp * rsqrtf(fmaf(S, S, c2s2)), acc2);
+      }
+      J = fmaf(0.78539816f, acc2, J);
+    }
+  }
+  return phi < 0.0f ? -J : J;                        // odd in phi
+}
+
+// von Mises torus entropy (reference dists/clifford.py:21-31 `_von_mises_entropy`, :277-278): per circle
+//   h(kappa) = ln 2 pi + ln a + kappa - kappa b / a,   a = i0e(kappa) + 1e-7,  b = i1e(kappa) + 1e-7
+// summed over circles k >= 1.  i0e / i1e from the fp64 log I_v e^{-x} of special.cuh (the reference's are torch's fp32
+// Chebyshev fits: agreement ~1e-7 relative); the eps regularisation and the final arithmetic follow the reference.
+// dh/dkappa (optional) is the exact derivative of that regularised expression:
+//   a' = i1e - i0e,  b' = i0e - i1e (1 + 1/kappa):   h' = a'/a + 1 - b/a - kappa (b' a - b a') / a^2
+struct VmEntropy { float h, dh; };
+__device__ __forceinline__ VmEntropy vm_circle_entropy(float kappa_f) {
+  const double k = (double)kappa_f;
+  double i0e = 1.0, i1e = 0.0;
+  if (k > 0.0) { i0e = exp(log_ive(0.0, k)); i1e = exp(log_ive(1.0, k)); }
+  const double eps = (double)1e-7f;
+  const double a = (double)(float)(i0e) + eps, b = (double)(float)(i1e) + eps;   // the reference adds eps to fp32 values
+  VmEntropy o;
+  o.h = (float)(1.83787706640934548356 + log(a) + k - k * (b / a));
+  const double da = i1e - i0e, db = (k > 0.0) ? i0e - i1e * (1.0 + 1.0 / k) : 0.5;
+  o.dh = (float)(da / a + 1.0 - b / a - k * (db * a - b * da) / (a * a));
+  return o;
 }
 
 // Per-row input pointers, indexed by the bin k: either the global rows or their staged copies in
@@ -229,7 +336,9 @@ __device__ __forceinline__ bool clifford_phasor(const CliffordFwdParams& p, cons
     const float kap = __ldg(p.kappa + prow * p.kappa_row_stride + (long long)k * p.kappa_el_stride);
     PhiloxKey vkey = p.key;
     vkey.stream = 11;
-    th = src.loc[k] + von_mises_draw(kap, vkey, (uint64_t)idx);
+    const float phi = von_mises_draw(kap, vkey, (uint64_t)idx);
+    if (p.tp_signed) stg_stream1(p.tp_signed + idx, phi);     // the drawn offset, saved for the backward
+    th = src.loc[k] + phi;
     sincosf(th, &out.y, &out.x);
     return true;
   }
@@ -297,6 +406,20 @@ __device__ __forceinline__ void clifford_row_entropy(const CliffordFwdParams& p,
     const double l0 = log1p((double)fminf(fmaxf(c0, -1.0f + kEps), 1.0f - kEps));
     atomicAdd(p.log_prob + row, (float)((double)p.d * c.log_norm +
                                         (double)kap_row * ((double)(p.d - 1) * 0.69314718055994530942 + l0)));
+  }
+}
+
+// von Mises torus rows (kVonMisesRng, one concentration per row): the row entropy / KL to the uniform prior / dH/dkappa
+// of the sampled rows, the same arithmetic as vm_entropy_kernel, one row per thread of the whole launch (the launcher
+// requests them only when kappa_el_stride == 0)
+__device__ __forceinline__ void vm_fwd_row_entropies(const CliffordFwdParams& p, long long first, long long step) {
+  if (!(p.entropy || p.kl || p.dentropy)) return;
+  for (long long row = first; row < p.rows; row += step) {
+    const VmEntropy e = vm_circle_entropy(__ldg(p.kappa + (row % p.loc_rows) * p.kappa_row_stride));
+    const float h = (float)(p.d - 1) * e.h;
+    if (p.entropy) p.entropy[row] = h;
+    if (p.kl) p.kl[row] = (float)((double)(p.d - 1) * 1.83787706640934548356 - (double)h);
+    if (p.dentropy) p.dentropy[row] = (float)(p.d - 1) * e.dh;
   }
 }
 
@@ -407,6 +530,8 @@ clifford_fwd_kernel(const CliffordFwdParams p, const cplx* __restrict__ tw, cons
         clifford_row_entropy<LEAN || BIND>(p, row, fwd_row_kappa<LEAN || BIND>(p, row % p.loc_rows));
     }
   }
+  if constexpr (MODE == kVonMisesRng)
+    vm_fwd_row_entropies(p, (long long)blockIdx.x * blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x);
 
   // Row schedule.  Static: group g of CTA b takes rows b*G + g + i*stride.  Dynamic (sched != null, groups of
   // >= 32 threads): after its first row a group fetches the next unprocessed row from a global counter, which
@@ -771,6 +896,27 @@ __device__ __forceinline__ float clifford_bwd_element(const CliffordBwdParams& p
   return dth;
 }
 
+// Element k of the von Mises torus backward (src.tps = the offsets phi the forward drew): dL/dloc_k = dL/dtheta_k,
+// dL/dkappa_k = dL/dtheta_k * d phi_k / d kappa_k (implicit gradient, vm_dphi_dkappa).  ROWK: kap / b are the row's,
+// else the element's are read here.  Returns dL/dkappa_k; stores dL/dloc_k (and dL/dkappa_k unless ROWK).
+template <bool ROWK>
+__device__ __forceinline__ float vm_bwd_element(const CliffordBwdParams& p, const BwdRowSrc& src, long long row,
+                                                long long prow, int k, cplx Gk, float kap, float b, float inv_d) {
+  const long long idx = row * p.d + k;
+  const float phi = src.tps[k];
+  float s, c;
+  sincosf(src.loc[k] + phi, &s, &c);                 // theta as the forward formed it
+  const float dth = -inv_d * (s * Gk.x - c * Gk.y);   // -(2/n) Im(X_k conj(G_k))
+  if (!ROWK) {
+    kap = __ldg(p.kappa + prow * p.kappa_row_stride + (long long)k * p.kappa_el_stride);
+    b = vm_row_consts(kap).b;
+  }
+  const float dk = dth * vm_dphi_dkappa(phi, kap, b);
+  stg_stream1(p.dloc + idx, dth);
+  if (!ROWK) stg_stream1(p.dkappa + idx, dk);
+  return dk;
+}
+
 // Rows the forward sampled through the inverse-CDF table (device RNG, one concentration <= kIcdfKappaMax per row, d >= 512)
 // save the signed TABLE COORDINATE of every draw instead of copysign(t', s), and the backward differentiates
 // the table map itself: phase and d phase / d kappa from the row's cells (icdf_phi_and_dkappa) -- the exact pathwise
@@ -781,24 +927,27 @@ __device__ __forceinline__ float clifford_bwd_element(const CliffordBwdParams& p
 // still gains: 25.0 -> 31.9 % of the roofline; d = 2048: 27.6 -> 38.2 %.)
 // smem per group: staged rows (loc, tp_signed | tprime, gnoise; FAST: two) | value + derivative cells (table rows) |
 // exchange buffer | 32 floats reduction scratch + row constants | mbarrier
-template <int LOG2N, bool ROWK = true, bool FAST = false>
+template <int LOG2N, bool ROWK = true, bool FAST = false, bool VM = false>
 constexpr size_t clifford_bwd_smem_bytes() {
   using Pl = FftPlan<LOG2N>;
-  return (sizeof(cplx) * Pl::XCH + sizeof(float) * (32 + 2 * kBetaRowFloats) + sizeof(float) * (FAST ? 2 : 3) * Pl::N +
-          ((ROWK && clifford_saves_table_coord<LOG2N>()) ? 2 * sizeof(float4) * kIcdfCells : 0) + sizeof(uint64_t)) * Pl::GROUPS;
+  return (sizeof(cplx) * Pl::XCH + sizeof(float) * (32 + 2 * kBetaRowFloats) + sizeof(float) * ((FAST || VM) ? 2 : 3) * Pl::N +
+          ((!VM && ROWK && clifford_saves_table_coord<LOG2N>()) ? 2 * sizeof(float4) * kIcdfCells : 0) + sizeof(uint64_t)) * Pl::GROUPS;
 }
 
 // FAST: saved draws + TMA-staged element inputs (the training path: backward of a device-RNG rsample with 16-byte
 // aligned rows); the injected-draw and unstaged paths are compiled out.
-template <int LOG2N, bool ROWK, bool FAST = false>
+// VM: the von Mises torus family (cvb_clifford_vm_rsample_backward): the staged rows are loc and the saved offsets phi,
+// the row constant is 1 - A(kappa) (vm_row_consts) and the element is vm_bwd_element; the R2C transform of grad_z and
+// the row schedule are the power-spherical ones.
+template <int LOG2N, bool ROWK, bool FAST = false, bool VM = false>
 __global__ void __launch_bounds__(FftPlan<LOG2N>::THREADS, (FftPlan<LOG2N>::THREADS <= 128 ? clifford_bwd_min_blocks<LOG2N>() : 1))
 clifford_bwd_kernel(const CliffordBwdParams p, const cplx* __restrict__ tw, const float2* __restrict__ icdf) {
   pdl_wait_and_release();
   using Pl = FftPlan<LOG2N>;
   constexpr int d = Pl::N, T = Pl::T, E = Pl::E, G = Pl::GROUPS;
   constexpr uint32_t kRowBytes = d * sizeof(float);
-  constexpr bool TABLE = ROWK && clifford_saves_table_coord<LOG2N>();
-  constexpr int NSTAGE = FAST ? 2 : 3;
+  constexpr bool TABLE = !VM && ROWK && clifford_saves_table_coord<LOG2N>();
+  constexpr int NSTAGE = (FAST || VM) ? 2 : 3;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int group = threadIdx.x / T, t = threadIdx.x % T;
   // layout: [G x staged rows][G x (value cells | derivative cells)][G x xch][G x scratch][G x mbarrier]
@@ -814,7 +963,7 @@ clifford_bwd_kernel(const CliffordBwdParams p, const cplx* __restrict__ tw, cons
   uint64_t* bar = reinterpret_cast<uint64_t*>(after_stage + (sizeof(cplx) * Pl::XCH + sizeof(float) * kScratch) * (size_t)G) + group;
   const long long stride = (long long)gridDim.x * G;
   const bool staged = FAST ? true : (p.staged != 0);
-  const bool saved = FAST ? true : (p.tp_signed != nullptr);
+  const bool saved = (FAST || VM) ? true : (p.tp_signed != nullptr);
 
   // bulk copies of one row's element inputs (thread 0 of the group); they land while grad_z is transformed
   auto issue = [&](long long row) {
@@ -857,7 +1006,9 @@ clifford_bwd_kernel(const CliffordBwdParams p, const cplx* __restrict__ tw, cons
     float* rc = rowconst + (parity ? kBetaRowFloats : 0);
     // a row the forward sampled through the table (same predicate as clifford_fwd_kernel; uniform over the group)
     const bool table_row = TABLE && saved && valid && kap_row >= 0.0f && (kap_row + kEps <= kIcdfKappaMax);
-    if (TABLE && table_row) {
+    if constexpr (VM) {
+      if (ROWK && t == 0) rc[0] = vm_row_consts(kap_row).b;
+    } else if (TABLE && table_row) {
       // every thread left the previous row's element loop (its closing barriers) before these are overwritten
       icdf_build_row_both(cells, dcells, kap_row + kEps, icdf, t, T);
     } else if (ROWK) {
@@ -924,7 +1075,8 @@ clifford_bwd_kernel(const CliffordBwdParams p, const cplx* __restrict__ tw, cons
         const int k = t + e * T;
         float dk = 0.f;
         if (valid && k != 0) {
-          clifford_bwd_element<ROWK, BetaGradRowShared, FAST>(p, src, row, prow, k, xch[pad16(k)], bc, 1.0f / (float)d, dk);
+          if constexpr (VM) dk = vm_bwd_element<ROWK>(p, src, row, prow, k, xch[pad16(k)], kap_row, rc[0], 1.0f / (float)d);
+          else clifford_bwd_element<ROWK, BetaGradRowShared, FAST>(p, src, row, prow, k, xch[pad16(k)], bc, 1.0f / (float)d, dk);
         } else if (valid) {
           stg_stream1(p.dloc + row * d, 0.0f);
           if (!ROWK) stg_stream1(p.dkappa + row * d, 0.0f);
@@ -1014,9 +1166,59 @@ __device__ __forceinline__ void clifford_lp_element(const CliffordLogProbParams&
   }
 }
 
+// Element k of the von Mises torus log_prob: kappa cos(a_k - loc_k) - ln(2 pi I0(kappa)) for circles k >= 1 (circle 0 adds
+// nothing and gets zero gradients), a_k = angle(F_k), angle(0) = 0.  Evaluated as kappa (cos d - 1) - lnk with
+// cos d - 1 = -|u - m|^2 / 2 (u = F_k / |F_k|, m = (cos loc, sin loc)) and lnk = ln 2 pi + log_ive(0, kappa): the two
+// kappa-sized halves cancel in closed form instead of in fp32.  d/dloc = kappa sin(a - loc), d/dkappa = cos(a - loc) - A
+// = (cos d - 1) + b, d/dF = kappa (m - (u.m) u) / |F|.  ROWK: kap / lnk / b are the row's, else the element's.
+template <bool ROWK>
+__device__ __forceinline__ void vm_lp_element(const CliffordLogProbParams& p, long long row, long long prow, int k, cplx Fk,
+                                              float loc_k, float kap, float lnk, float b, float& acc, float& dk_acc) {
+  if (k == 0) {
+    if (p.dlp_dF) reinterpret_cast<float2*>(p.dlp_dF)[row * p.d] = make_float2(0.f, 0.f);
+    if (p.dlp_dloc) {
+      p.dlp_dloc[row * p.d] = 0.f;
+      if (!ROWK) p.dlp_dkappa[row * p.d] = 0.f;
+    }
+    return;
+  }
+  if (!ROWK) {
+    kap = __ldg(p.kappa + prow * p.kappa_row_stride + (long long)k * p.kappa_el_stride);
+    const VmRowConsts c = vm_row_consts(kap);
+    lnk = c.lnk;
+    b = c.b;
+  }
+  const float mag2 = fmaf(Fk.x, Fk.x, Fk.y * Fk.y);
+  float ca = 1.0f, sa = 0.0f;
+  if (mag2 > 0.f) {
+    const float ri = rsqrtf(mag2);
+    ca = Fk.x * ri;
+    sa = Fk.y * ri;
+  }
+  float sl, cl;
+  sincosf(loc_k, &sl, &cl);
+  const float dc = ca - cl, ds = sa - sl;
+  const float cm1 = -0.5f * fmaf(dc, dc, ds * ds);            // cos(a - loc) - 1
+  acc += fmaf(kap, cm1, -lnk);
+  if (p.dlp_dF) {
+    float2 gF = make_float2(0.f, 0.f);
+    if (mag2 > 0.f) {
+      const float dot = fmaf(cl, ca, sl * sa), c = kap * rsqrtf(mag2);
+      gF = make_float2(c * fmaf(-dot, ca, cl), c * fmaf(-dot, sa, sl));
+    }
+    reinterpret_cast<float2*>(p.dlp_dF)[row * p.d + k] = gF;
+  }
+  if (p.dlp_dloc) {
+    stg_stream1(p.dlp_dloc + row * p.d + k, kap * fmaf(cl, sa, -sl * ca));
+    const float dkv = cm1 + b;
+    if (ROWK) dk_acc += dkv; else stg_stream1(p.dlp_dkappa + row * p.d + k, dkv);
+  }
+}
+
 constexpr int kLpConstCache = 256;   // rows per group whose log-normaliser constants are precomputed
 
-template <int LOG2N, bool ROWK, bool FWD_ONLY = false>
+// VM: the von Mises torus family (vm_lp_element; row constants (lnk, 1 - A) in place of (log C, dlog C / dkappa)).
+template <int LOG2N, bool ROWK, bool FWD_ONLY = false, bool VM = false>
 __global__ void __launch_bounds__(FftPlan<LOG2N>::THREADS, (FftPlan<LOG2N>::THREADS <= 128 ? ((FWD_ONLY && LOG2N <= 9) ? 5 : 4) : 1))
 clifford_log_prob_kernel(const CliffordLogProbParams p, const cplx* __restrict__ tw) {
   pdl_wait_and_release();
@@ -1037,8 +1239,13 @@ clifford_log_prob_kernel(const CliffordLogProbParams p, const cplx* __restrict__
     for (int i = t; i < kLpConstCache; i += T) {
       const long long row = first_row + (long long)i * stride;
       if (row < p.rows) {
-        const PsConsts c = ps_consts((double)__ldg(p.kappa + (row % p.loc_rows) * p.kappa_row_stride), 0.5);
-        ccache[i] = make_float2((float)c.log_norm, (float)c.dlog_norm);
+        if constexpr (VM) {
+          const VmRowConsts c = vm_row_consts(__ldg(p.kappa + (row % p.loc_rows) * p.kappa_row_stride));
+          ccache[i] = make_float2(c.lnk, c.b);
+        } else {
+          const PsConsts c = ps_consts((double)__ldg(p.kappa + (row % p.loc_rows) * p.kappa_row_stride), 0.5);
+          ccache[i] = make_float2((float)c.log_norm, (float)c.dlog_norm);
+        }
       }
     }
   }
@@ -1065,13 +1272,17 @@ clifford_log_prob_kernel(const CliffordLogProbParams p, const cplx* __restrict__
       if (iter < kLpConstCache) {
         const float2 c = ccache[iter];
         logc = c.x; dlogc = c.y;
+      } else if constexpr (VM) {
+        const VmRowConsts c = vm_row_consts(kap_row);
+        logc = c.lnk;
+        dlogc = c.b;
       } else {
         const PsConsts c = ps_consts((double)kap_row, 0.5);
         logc = (float)c.log_norm;
         dlogc = (float)c.dlog_norm;
       }
     }
-    if constexpr (FWD_ONLY && ROWK) {
+    if constexpr (FWD_ONLY && ROWK && !VM) {
       // Evaluation with one concentration per row: the element is ~20 instructions (MUFU sincos / rsqrt / lg2), so it is
       // unrolled over the registers that already hold F[k] and loc[k] -- no round trip through shared memory, no barrier,
       // no branch per bin (angle(0) = 0 by a select); sum_k (log C + kappa l_k) = d log C + kappa sum_k l_k per thread.
@@ -1100,7 +1311,11 @@ clifford_log_prob_kernel(const CliffordLogProbParams p, const cplx* __restrict__
 #pragma unroll 2
     for (int e = 0; e < E; ++e) {
       const int k = t + e * T;
-      if (valid) clifford_lp_element<ROWK, FWD_ONLY>(p, row, prow, k, xch[pad16(k)], locs[k], kap_row, logc, dlogc, acc, dk_acc);
+      if constexpr (VM) {
+        if (valid) vm_lp_element<ROWK>(p, row, prow, k, xch[pad16(k)], locs[k], kap_row, logc, dlogc, acc, dk_acc);
+      } else {
+        if (valid) clifford_lp_element<ROWK, FWD_ONLY>(p, row, prow, k, xch[pad16(k)], locs[k], kap_row, logc, dlogc, acc, dk_acc);
+      }
     }
     const float tot = group_sum<LOG2N>(acc, scratch, t);
     float dk_tot = 0.f;
@@ -1151,6 +1366,8 @@ clifford_fwd_generic_kernel(const CliffordFwdParams p) {
   cplx* X = smem + n;
   constexpr bool PS = (MODE == kPsInjected || MODE == kPsRng);
   fill_twiddles(tw, n);
+  if constexpr (MODE == kVonMisesRng)
+    vm_fwd_row_entropies(p, (long long)blockIdx.x * blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x);
   for (long long row = blockIdx.x; row < p.rows; row += gridDim.x) {
     const long long prow = row % p.loc_rows;
     float kap_row = 1.0f;
@@ -1189,8 +1406,8 @@ clifford_fwd_generic_kernel(const CliffordFwdParams p) {
   if (MODE == kPsRng || MODE == kUniformRng || MODE == kUnitaryRng || MODE == kVonMisesRng) rng_launch_done(p.key);
 }
 
-// smem: tw[n] cplx, g[n] float, scratch[32] float
-template <bool ROWK>
+// smem: tw[n] cplx, g[n] float, scratch[32] float.  VM: the von Mises torus family (vm_bwd_element).
+template <bool ROWK, bool VM = false>
 __global__ void __launch_bounds__(kGenericThreads)
 clifford_bwd_generic_kernel(const CliffordBwdParams p) {
   extern __shared__ cplx smem[];
@@ -1207,6 +1424,8 @@ clifford_bwd_generic_kernel(const CliffordBwdParams p) {
     const float kap_raw = __ldg(p.kappa + prow * p.kappa_row_stride);
     const float kap_row = head_kappa(p.head, kap_raw);
     BetaGradRow bc(0.5f + (kap_row + kEps), 0.5f);
+    float vm_b = 1.0f;
+    if constexpr (VM) { if (ROWK) vm_b = vm_row_consts(kap_row).b; }
     BwdRowSrc gsrc;
     gsrc.loc = p.loc + prow * d;
     gsrc.tps = p.tp_signed ? p.tp_signed + row * d : nullptr;
@@ -1229,7 +1448,8 @@ clifford_bwd_generic_kernel(const CliffordBwdParams p) {
         if (m >= n) m -= n;
       }
       float dk = 0.f;
-      clifford_bwd_element<ROWK>(p, gsrc, row, prow, k, make_float2((float)gr, (float)gi), bc, 1.0f / (float)d, dk);
+      if constexpr (VM) dk = vm_bwd_element<ROWK>(p, gsrc, row, prow, k, make_float2((float)gr, (float)gi), kap_row, vm_b, 1.0f / (float)d);
+      else clifford_bwd_element<ROWK>(p, gsrc, row, prow, k, make_float2((float)gr, (float)gi), bc, 1.0f / (float)d, dk);
       dk_sum += dk;
     }
     if (ROWK) {
@@ -1239,7 +1459,7 @@ clifford_bwd_generic_kernel(const CliffordBwdParams p) {
   }
 }
 
-template <bool ROWK>
+template <bool ROWK, bool VM = false>
 __global__ void __launch_bounds__(kGenericThreads)
 clifford_log_prob_generic_kernel(const CliffordLogProbParams p) {
   extern __shared__ cplx smem[];
@@ -1255,7 +1475,13 @@ clifford_log_prob_generic_kernel(const CliffordLogProbParams p) {
     __syncthreads();
     const float kap_row = __ldg(p.kappa + prow * p.kappa_row_stride);
     float logc = 0.f, dlogc = 0.f;
-    if (ROWK) {
+    if constexpr (VM) {
+      if (ROWK) {
+        const VmRowConsts c = vm_row_consts(kap_row);
+        logc = c.lnk;
+        dlogc = c.b;
+      }
+    } else if (ROWK) {
       const PsConsts c = ps_consts((double)kap_row, 0.5);
       logc = (float)c.log_norm;
       dlogc = (float)c.dlog_norm;
@@ -1272,8 +1498,12 @@ clifford_log_prob_generic_kernel(const CliffordLogProbParams p) {
         if (m >= n) m -= n;
       }
       if (k == 0) fi = 0.0;
-      clifford_lp_element<ROWK>(p, row, prow, k, make_float2((float)fr, (float)fi), p.loc[prow * d + k], kap_row, logc, dlogc,
-                                acc, dk_acc);
+      if constexpr (VM)
+        vm_lp_element<ROWK>(p, row, prow, k, make_float2((float)fr, (float)fi), p.loc[prow * d + k], kap_row, logc, dlogc,
+                            acc, dk_acc);
+      else
+        clifford_lp_element<ROWK>(p, row, prow, k, make_float2((float)fr, (float)fi), p.loc[prow * d + k], kap_row, logc, dlogc,
+                                  acc, dk_acc);
     }
     const float tot = block_sum_256(acc, scratch);
     float dk_tot = 0.f;
@@ -1336,25 +1566,6 @@ static __global__ void ps_entropy_kernel(const EntropyParams p) {
   }
 }
 
-// von Mises torus entropy (reference dists/clifford.py:21-31 `_von_mises_entropy`, :277-278): per circle
-//   h(kappa) = ln 2 pi + ln a + kappa - kappa b / a,   a = i0e(kappa) + 1e-7,  b = i1e(kappa) + 1e-7
-// summed over circles k >= 1.  i0e / i1e from the fp64 log I_v e^{-x} of special.cuh (the reference's are torch's fp32
-// Chebyshev fits: agreement ~1e-7 relative); the eps regularisation and the final arithmetic follow the reference.
-// dh/dkappa (optional) is the exact derivative of that regularised expression:
-//   a' = i1e - i0e,  b' = i0e - i1e (1 + 1/kappa):   h' = a'/a + 1 - b/a - kappa (b' a - b a') / a^2
-struct VmEntropy { float h, dh; };
-__device__ __forceinline__ VmEntropy vm_circle_entropy(float kappa_f) {
-  const double k = (double)kappa_f;
-  double i0e = 1.0, i1e = 0.0;
-  if (k > 0.0) { i0e = exp(log_ive(0.0, k)); i1e = exp(log_ive(1.0, k)); }
-  const double eps = (double)1e-7f;
-  const double a = (double)(float)(i0e) + eps, b = (double)(float)(i1e) + eps;   // the reference adds eps to fp32 values
-  VmEntropy o;
-  o.h = (float)(1.83787706640934548356 + log(a) + k - k * (b / a));
-  const double da = i1e - i0e, db = (k > 0.0) ? i0e - i1e * (1.0 + 1.0 / k) : 0.5;
-  o.dh = (float)(da / a + 1.0 - b / a - k * (db * a - b * da) / (a * a));
-  return o;
-}
 // One warp per row; kappa addressed like the samplers' (el_stride 0: one concentration per row).
 static __global__ void vm_entropy_kernel(const EntropyParams p) {
   const int lane = threadIdx.x & 31;

@@ -50,6 +50,8 @@ clifford_fwd_small_kernel(const CliffordFwdParams p, const int RT) {
   cplx* X = tw + ((n + 1) & ~1);                             // [k = 0 .. nph][r]; slot k = 0 holds (dc, nyquist)
   constexpr bool PS = (MODE == kPsInjected || MODE == kPsRng);
   fill_twiddles(tw, n);
+  if constexpr (MODE == kVonMisesRng)
+    vm_fwd_row_entropies(p, (long long)blockIdx.x * blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x);
   const long long tiles = (p.rows + RT - 1) / RT;
   const float inv_n = 1.0f / (float)n;
   for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
@@ -170,7 +172,8 @@ __device__ __forceinline__ void small_rows_dft(const float* __restrict__ src, lo
   __syncthreads();
 }
 
-template <bool ROWK>
+// VM: the von Mises torus family (saved offsets phi in tp_signed; row constant 1 - A(kappa) in rowconst[0]).
+template <bool ROWK, bool VM = false>
 __global__ void __launch_bounds__(kSmallThreads)
 clifford_bwd_small_kernel(const CliffordBwdParams p, const int RT) {
   extern __shared__ __align__(16) unsigned char smem_small[];
@@ -192,9 +195,13 @@ clifford_bwd_small_kernel(const CliffordBwdParams p, const int RT) {
       for (int r = threadIdx.x; r < RT; r += kSmallThreads) {
         if (row0 + r < p.rows) {
           const float kap = head_kappa(p.head, __ldg(p.kappa + ((row0 + r) % p.loc_rows) * p.kappa_row_stride));
-          const BetaGradConsts c(0.5f + (kap + kEps), 0.5f);
           float* o = rowconst + r * kSmallRowConst;
-          o[0] = c.alpha; o[1] = c.beta; o[2] = c.total; o[3] = c.psi_alpha; o[4] = c.psi_total; o[5] = c.log_alpha; o[6] = c.log_total;
+          if constexpr (VM) {
+            o[0] = vm_row_consts(kap).b;
+          } else {
+            const BetaGradConsts c(0.5f + (kap + kEps), 0.5f);
+            o[0] = c.alpha; o[1] = c.beta; o[2] = c.total; o[3] = c.psi_alpha; o[4] = c.psi_total; o[5] = c.log_alpha; o[6] = c.log_total;
+          }
         }
       }
     }
@@ -218,7 +225,10 @@ clifford_bwd_small_kernel(const CliffordBwdParams p, const int RT) {
           continue;
         }
         float dk = 0.f;
-        clifford_bwd_element<ROWK>(p, src, row, prow, k, G[k * XP + r], bc, 1.0f / (float)d, dk);
+        if constexpr (VM)
+          dk = vm_bwd_element<ROWK>(p, src, row, prow, k, G[k * XP + r], __ldg(p.kappa + prow * p.kappa_row_stride),
+                                    rowconst[r * kSmallRowConst], 1.0f / (float)d);
+        else clifford_bwd_element<ROWK>(p, src, row, prow, k, G[k * XP + r], bc, 1.0f / (float)d, dk);
         dk_sum += dk;
       }
     }
@@ -242,7 +252,8 @@ inline size_t clifford_lp_small_smem(int d, int rt) {
          sizeof(float) * 2 * (size_t)kSmallThreads + sizeof(float2) * (size_t)rt;
 }
 
-template <bool ROWK>
+// VM: the von Mises torus family (vm_lp_element; consts[r] = (lnk, 1 - A)).
+template <bool ROWK, bool VM = false>
 __global__ void __launch_bounds__(kSmallThreads)
 clifford_lp_small_kernel(const CliffordLogProbParams p, const int RT) {
   extern __shared__ __align__(16) unsigned char smem_small[];
@@ -262,8 +273,13 @@ clifford_lp_small_kernel(const CliffordLogProbParams p, const int RT) {
     if (ROWK) {
       for (int r = threadIdx.x; r < RT; r += kSmallThreads) {
         if (row0 + r < p.rows) {
-          const PsConsts c = ps_consts((double)__ldg(p.kappa + ((row0 + r) % p.loc_rows) * p.kappa_row_stride), 0.5);
-          consts[r] = make_float2((float)c.log_norm, (float)c.dlog_norm);
+          if constexpr (VM) {
+            const VmRowConsts c = vm_row_consts(__ldg(p.kappa + ((row0 + r) % p.loc_rows) * p.kappa_row_stride));
+            consts[r] = make_float2(c.lnk, c.b);
+          } else {
+            const PsConsts c = ps_consts((double)__ldg(p.kappa + ((row0 + r) % p.loc_rows) * p.kappa_row_stride), 0.5);
+            consts[r] = make_float2((float)c.log_norm, (float)c.dlog_norm);
+          }
         }
       }
     }
@@ -278,7 +294,8 @@ clifford_lp_small_kernel(const CliffordLogProbParams p, const int RT) {
       for (int k = kk; k < d; k += TPR) {
         cplx Fk = F[k * XP + r];
         if (k == 0) Fk.y = 0.0f;
-        clifford_lp_element<ROWK>(p, row, prow, k, Fk, __ldg(p.loc + prow * d + k), kap_row, c.x, c.y, acc, dk_acc);
+        if constexpr (VM) vm_lp_element<ROWK>(p, row, prow, k, Fk, __ldg(p.loc + prow * d + k), kap_row, c.x, c.y, acc, dk_acc);
+        else clifford_lp_element<ROWK>(p, row, prow, k, Fk, __ldg(p.loc + prow * d + k), kap_row, c.x, c.y, acc, dk_acc);
       }
     }
     part[kk * RT + r] = acc;

@@ -114,12 +114,35 @@ CVB_API int cvb_ps_entropy_kl(const float* kappa, long long kappa_row_stride, in
 /* CliffordTorusDistribution.rsample (dists/clifford.py:261-275; scripts/sample_viz.py:55-64 restates it): phases
  * theta = loc + VonMises(0, kappa) drawn on the device with Best & Fisher's rejection (the algorithm behind
  * torch.distributions.VonMises.sample, which the reference calls at :262), then the same Hermitian spectrum -> C2R
- * inverse FFT.  kappa addressed like cvb_clifford_ps_rsample's.  Not reparameterised (no backward), like the
- * reference.  (The reference's own method stops at its Hermitian-symmetry assert, :274; this entry point is the
- * working version of what it computes.) */
+ * inverse FFT.  kappa addressed like cvb_clifford_ps_rsample's.  Forward only; cvb_clifford_vm_rsample_kl draws the
+ * same z and saves what its backward needs.  (The reference's own method stops at its Hermitian-symmetry assert, :274;
+ * this entry point is the working version of what it computes.) */
 CVB_API int cvb_clifford_vm_rsample(const float* loc, const float* kappa, long long kappa_row_stride, int kappa_el_stride,
                                     long long loc_rows, unsigned long long seed, unsigned long long offset, float* z,
                                     long long rows, int d, void* stream);
+/* cvb_clifford_vm_rsample with a reparameterised backward: bitwise the same z for the same (seed, offset).  phi
+ * (rows, d) optional: the drawn offsets theta_k - loc_k, saved for cvb_clifford_vm_rsample_backward (opaque; element 0
+ * unwritten).  entropy / kl / dentropy (rows) optional, only with kappa_el_stride == 0: the row values that
+ * cvb_clifford_vm_entropy gives, and kl = (d-1) ln 2 pi - entropy (the KL to CliffordTorusUniform), from the same launch. */
+CVB_API int cvb_clifford_vm_rsample_kl(const float* loc, const float* kappa, long long kappa_row_stride, int kappa_el_stride,
+                                       long long loc_rows, unsigned long long seed, unsigned long long offset, float* z,
+                                       float* phi, float* entropy, float* kl, float* dentropy, long long rows, int d,
+                                       void* stream);
+/* Backward of cvb_clifford_vm_rsample_kl, the implicit reparameterisation gradient of the von Mises draws: phi from the
+ * forward of the SAME (loc, kappa, rows, d).  dL/dtheta_k = -(1/d) Im(e^{i theta_k} conj(G_k)), G = rfft(grad_z);
+ * dloc (rows, d) = dL/dtheta (circle 0: 0); dkappa = dL/dtheta_k * d phi_k / d kappa_k, (rows) row sums when
+ * kappa_el_stride == 0, else (rows, d). */
+CVB_API int cvb_clifford_vm_rsample_backward(const float* grad_z, const float* loc, const float* kappa,
+                                             long long kappa_row_stride, int kappa_el_stride, long long loc_rows,
+                                             const float* phi, float* dloc, float* dkappa, long long rows, int d,
+                                             void* stream);
+/* CliffordTorusDistribution.log_prob: value (rows, 2d), a_k = angle(rfft(value)_k) ->
+ * log_prob (rows) = sum_{k=1}^{d-1} kappa_k cos(a_k - loc_k) - ln(2 pi I0(kappa_k)) (the circles of the entropy and of
+ * the uniform prior).  Optional derivative outputs as cvb_clifford_ps_log_prob's (give dlp_dloc and dlp_dkappa both or
+ * neither; dlp_dF (rows, d) complex); circle 0 gets zeros. */
+CVB_API int cvb_clifford_vm_log_prob(const float* value, const float* loc, const float* kappa, long long kappa_row_stride,
+                                     int kappa_el_stride, long long loc_rows, float* log_prob, float* dlp_dloc,
+                                     float* dlp_dkappa, float* dlp_dF, long long rows, int d, void* stream);
 
 /* CliffordTorusUniform.rsample (dists/clifford.py:228-236) and the shared "phases -> real vector with
  * unit-magnitude spectrum" map.  phases (rows, d) are multiplied by phase_scale (2*pi for uniform u);
