@@ -1,15 +1,10 @@
 // C ABI entry points for the Clifford-torus kernels (include/clifford_b200.h).
-#include <cstdlib>
-#include "launch.cuh"
-#include "clifford_kernels.cuh"
-#include "clifford_small.cuh"
+#include "clifford_launch.cuh"
 #include "../../include/clifford_b200.h"
 
 using namespace cvb;
 
 namespace {
-
-constexpr size_t kGenericSmemLimit = 200 * 1024;
 
 template <int LOG2N, bool ROWK, bool FAST = false, bool VM = false>
 int launch_bwd_fast(const CliffordBwdParams& p, cudaStream_t st) {
@@ -20,50 +15,23 @@ int launch_bwd_fast(const CliffordBwdParams& p, cudaStream_t st) {
   const cplx* tw = device_twiddles();
   const float2* icdf = device_icdf_table();
   if (!tw || !icdf) return kCudaError;
-  const size_t smem = clifford_bwd_smem_bytes<LOG2N, ROWK, FAST, VM>();
-  auto kern = clifford_bwd_kernel<LOG2N, ROWK, FAST, VM>;
-  int grid = 0;
-  const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
   CliffordBwdParams q = p;
-  static const bool static_sched = getenv("CVB_STATIC_SCHEDULE") != nullptr;
-  q.sched = (Pl::GROUPS == 1 && !static_sched && work > grid) ? next_sched_slot() : nullptr;   // dynamic rows when CTAs loop
-  launch_pdl(kern, grid, Pl::THREADS, smem, st, q, tw, icdf);
-  return check_launch("clifford_bwd_kernel");
+  // dynamic rows only with one row per CTA
+  return launch_persistent_pdl(clifford_bwd_kernel<LOG2N, ROWK, FAST, VM>, "clifford_bwd_kernel", Pl::THREADS,
+                               clifford_bwd_smem_bytes<LOG2N, ROWK, FAST, VM>(), (p.rows + Pl::GROUPS - 1) / Pl::GROUPS,
+                               Pl::GROUPS == 1 ? &q.sched : nullptr, st, q, tw, icdf);
 }
 
 template <bool ROWK, bool VM = false>
 int dispatch_bwd(const CliffordBwdParams& p_in, cudaStream_t st) {
   CliffordBwdParams p = p_in;
   p.staged = aligned(p.loc, 16) && (!p.tp_signed || aligned(p.tp_signed, 16)) && (!p.tprime || aligned(p.tprime, 16)) &&
-             (!p.gnoise || aligned(p.gnoise, 16)) && getenv("CVB_NO_TMA") == nullptr;
-  const bool fast = is_pow2(p.d) && p.d >= 16 && p.d <= 8192 && aligned(p.grad_z, 8);
-  if (fast) {
-    switch (ilog2(p.d)) {
-#define CVB_CASE(L) case L: return launch_bwd_fast<L, ROWK, false, VM>(p, st);
-      CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-      CVB_CASE(13)
-#undef CVB_CASE
-    }
-  }
-  static const bool no_small = getenv("CVB_NO_SMALL_ROWS") != nullptr;
-  if (2 * p.d <= kSmallMaxN && !no_small) {
-    const int rt = small_rows_per_tile(p.rows, sm_count(), [&](int r) { return clifford_bwd_small_smem(p.d, r); });
-    const size_t smem_s = clifford_bwd_small_smem(p.d, rt);
-    auto kern_s = clifford_bwd_small_kernel<ROWK, VM>;
-    int grid_s = 0;
-    if (int rc = persistent_grid(kern_s, kSmallThreads, smem_s, (p.rows + rt - 1) / rt, &grid_s)) return rc;
-    kern_s<<<grid_s, kSmallThreads, smem_s, st>>>(p, rt);
-    return check_launch("clifford_bwd_small_kernel");
-  }
+             (!p.gnoise || aligned(p.gnoise, 16));
   const int n = 2 * p.d;
-  const size_t smem = sizeof(cplx) * n + sizeof(float) * (n + 32);
-  CVB_REQUIRE(smem <= kGenericSmemLimit, kUnsupported, "clifford backward: d=%d too large for the direct-DFT path", p.d);
-  auto kern = clifford_bwd_generic_kernel<ROWK, VM>;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, kGenericThreads, smem, p.rows, &grid)) return rc;
-  kern<<<grid, kGenericThreads, smem, st>>>(p);
-  return check_launch("clifford_bwd_generic_kernel");
+  return dispatch_clifford(
+      "clifford backward", p, n, p.grad_z, [&](auto L) { return launch_bwd_fast<decltype(L)::value, ROWK, false, VM>(p, st); },
+      clifford_bwd_small_kernel<ROWK, VM>, [&](int r) { return clifford_bwd_small_smem(p.d, r); },
+      clifford_bwd_generic_kernel<ROWK, VM>, sizeof(cplx) * n + sizeof(float) * (n + 32), st);
 }
 
 }  // namespace

@@ -1,47 +1,25 @@
 // C ABI entry points for the Clifford-torus kernels (include/clifford_b200.h).
-#include <cstdlib>
-#include "launch.cuh"
-#include "clifford_kernels.cuh"
-#include "clifford_small.cuh"
+#include "clifford_launch.cuh"
 #include "../../include/clifford_b200.h"
 
 using namespace cvb;
 
 namespace {
 
-constexpr size_t kGenericSmemLimit = 200 * 1024;
-
 template <int LOG2N, int MODE, bool ROWK, bool LEAN = false>
 int launch_fwd_fast(const CliffordFwdParams& p, cudaStream_t st) {
-  using Pl = FftPlan<LOG2N>;
-  const cplx* tw = device_twiddles();
-  const float2* icdf = device_icdf_table();
-  if (!tw || !icdf) return kCudaError;
-  const size_t smem = clifford_fwd_smem_bytes<LOG2N, MODE>();
-  auto kern = clifford_fwd_kernel<LOG2N, MODE, ROWK, false, LEAN>;
-  int grid = 0;
-  const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
-  if constexpr (LEAN) {
-    // (only reachable when the kernel is built for 7 resident CTAs / SM, -DCVB_FWD_LEAN_MINB=7: they won 2-3 % once a CTA
-    // looped over >= 8 rows, but the longer row latency cost 1-2 % when a CTA only gets 3-5 rows (B = 4096 at d = 2048);
-    // the default build is capped for 6, see clifford_kernels.cuh)
-    const int sms = sm_count();
-    if (grid == sms * 7) {
-      const double rows_per_cta = (double)work / (double)grid;
-      if (rows_per_cta > 2.0 && rows_per_cta < 6.0) grid = sms * 6;
-    }
-  }
-  static const bool static_sched = getenv("CVB_STATIC_SCHEDULE") != nullptr;
-  const bool dynamic = !static_sched && work > grid;                         // dynamic rows only when CTAs loop
   if constexpr (MODE == kPsRng && ROWK && !LEAN) {
     // plain forward sampling: the specialised variant (no optional outputs, staged inputs)
     if (!p.tp_signed && !p.log_prob && p.staged && !p.head.on) return launch_fwd_fast<LOG2N, MODE, ROWK, true>(p, st);
   }
+  using Pl = FftPlan<LOG2N>;
+  const cplx* tw = device_twiddles();
+  const float2* icdf = device_icdf_table();
+  if (!tw || !icdf) return kCudaError;
   CliffordFwdParams q = p;
-  q.sched = dynamic ? next_sched_slot() : nullptr;
-  launch_pdl(kern, grid, Pl::THREADS, smem, st, q, tw, icdf);
-  return check_launch("clifford_fwd_kernel");
+  return launch_persistent_pdl(clifford_fwd_kernel<LOG2N, MODE, ROWK, false, LEAN>, "clifford_fwd_kernel", Pl::THREADS,
+                               clifford_fwd_smem_bytes<LOG2N, MODE>(), (p.rows + Pl::GROUPS - 1) / Pl::GROUPS, &q.sched,
+                               st, q, tw, icdf);
 }
 
 template <int LOG2N, int MODE>
@@ -50,65 +28,29 @@ int launch_fwd_bind(const CliffordFwdParams& p, cudaStream_t st) {
   const cplx* tw = device_twiddles();
   const float2* icdf = device_icdf_table();
   if (!tw || !icdf) return kCudaError;
-  const size_t smem = clifford_fwd_smem_bytes<LOG2N, MODE, true>();
-  auto kern = clifford_fwd_kernel<LOG2N, MODE, true, true>;
-  int grid = 0;
-  const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
   CliffordFwdParams q = p;
-  static const bool static_sched = getenv("CVB_STATIC_SCHEDULE") != nullptr;
-  q.sched = (!static_sched && work > grid) ? next_sched_slot() : nullptr;
-  launch_pdl(kern, grid, Pl::THREADS, smem, st, q, tw, icdf);
-  return check_launch("clifford_fwd_kernel<bind>");
+  return launch_persistent_pdl(clifford_fwd_kernel<LOG2N, MODE, true, true>, "clifford_fwd_kernel<bind>", Pl::THREADS,
+                               clifford_fwd_smem_bytes<LOG2N, MODE, true>(), (p.rows + Pl::GROUPS - 1) / Pl::GROUPS,
+                               &q.sched, st, q, tw, icdf);
 }
 
 template <int MODE>
 int dispatch_fwd_bind(const CliffordFwdParams& p_in, cudaStream_t st) {
   CliffordFwdParams p = p_in;
-  p.staged = aligned(p.loc, 16) && (!p.tprime || aligned(p.tprime, 16)) && (!p.gnoise || aligned(p.gnoise, 16)) &&
-             getenv("CVB_NO_TMA") == nullptr;
-  switch (ilog2(p.d)) {
-#define CVB_CASE(L) case L: return launch_fwd_bind<L, MODE>(p, st);
-    CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-    CVB_CASE(13)
-#undef CVB_CASE
-  }
-  return kUnsupported;
+  p.staged = aligned(p.loc, 16) && (!p.tprime || aligned(p.tprime, 16)) && (!p.gnoise || aligned(p.gnoise, 16));
+  return with_int<4, 13>(ilog2(p.d), [&](auto L) { return launch_fwd_bind<decltype(L)::value, MODE>(p, st); });
 }
 
 template <int MODE, bool ROWK>
 int dispatch_fwd(const CliffordFwdParams& p_in, cudaStream_t st) {
   CliffordFwdParams p = p_in;
   p.staged = (!p.loc || aligned(p.loc, 16)) && (!p.tprime || aligned(p.tprime, 16)) && (!p.gnoise || aligned(p.gnoise, 16)) &&
-             (!p.phases || aligned(p.phases, 16)) && getenv("CVB_NO_TMA") == nullptr;
-  const bool fast = is_pow2(p.d) && p.d >= 16 && p.d <= 8192 && p.n == 2 * p.d && aligned(p.z, 8);
-  if (fast) {
-    switch (ilog2(p.d)) {
-#define CVB_CASE(L) case L: return launch_fwd_fast<L, MODE, ROWK>(p, st);
-      CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-      CVB_CASE(13)
-#undef CVB_CASE
-    }
-  }
-  static const bool no_small = getenv("CVB_NO_SMALL_ROWS") != nullptr;    // A/B switch: the one-CTA-per-row direct DFT
-  if (p.n <= kSmallMaxN && !no_small) {
-    // short rows (the reference's default MNIST latents, per-token latents): a tile of rows per CTA
-    const int rt = small_rows_per_tile(p.rows, sm_count(), [&](int r) { return clifford_fwd_small_smem(p.n, r); });
-    const size_t smem_s = clifford_fwd_small_smem(p.n, rt);
-    auto kern_s = clifford_fwd_small_kernel<MODE, ROWK>;
-    int grid_s = 0;
-    if (int rc = persistent_grid(kern_s, kSmallThreads, smem_s, (p.rows + rt - 1) / rt, &grid_s)) return rc;
-    kern_s<<<grid_s, kSmallThreads, smem_s, st>>>(p, rt);
-    return check_launch("clifford_fwd_small_kernel");
-  }
+             (!p.phases || aligned(p.phases, 16));
   const int nph = (p.n - 1) / 2;
-  const size_t smem = sizeof(cplx) * ((size_t)p.n + nph + 1);
-  CVB_REQUIRE(smem <= kGenericSmemLimit, kUnsupported, "clifford rsample: length n=%d too large for the direct-DFT path", p.n);
-  auto kern = clifford_fwd_generic_kernel<MODE, ROWK>;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, kGenericThreads, smem, p.rows, &grid)) return rc;
-  kern<<<grid, kGenericThreads, smem, st>>>(p);
-  return check_launch("clifford_fwd_generic_kernel");
+  return dispatch_clifford(
+      "clifford rsample", p, p.n, p.z, [&](auto L) { return launch_fwd_fast<decltype(L)::value, MODE, ROWK>(p, st); },
+      clifford_fwd_small_kernel<MODE, ROWK>, [&](int r) { return clifford_fwd_small_smem(p.n, r); },
+      clifford_fwd_generic_kernel<MODE, ROWK>, sizeof(cplx) * ((size_t)p.n + nph + 1), st);
 }
 
 }  // namespace

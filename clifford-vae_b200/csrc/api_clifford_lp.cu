@@ -1,15 +1,10 @@
 // C ABI entry points for the Clifford-torus kernels (include/clifford_b200.h).
-#include "launch.cuh"
-#include <cstdlib>
-#include "clifford_kernels.cuh"
-#include "clifford_small.cuh"
+#include "clifford_launch.cuh"
 #include "../../include/clifford_b200.h"
 
 using namespace cvb;
 
 namespace {
-
-constexpr size_t kGenericSmemLimit = 200 * 1024;
 
 template <int LOG2N, bool ROWK, bool FWD_ONLY = false, bool VM = false>
 int launch_lp_fast(const CliffordLogProbParams& p, cudaStream_t st) {
@@ -21,43 +16,17 @@ int launch_lp_fast(const CliffordLogProbParams& p, cudaStream_t st) {
   if (!tw) return kCudaError;
   const size_t smem = sizeof(cplx) * Pl::XCH * Pl::GROUPS + sizeof(float) * 32 * Pl::GROUPS + sizeof(float2) * kLpConstCache * Pl::GROUPS +
                       sizeof(float) * Pl::N * Pl::GROUPS;
-  auto kern = clifford_log_prob_kernel<LOG2N, ROWK, FWD_ONLY, VM>;
-  int grid = 0;
-  const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
-  launch_pdl(kern, grid, Pl::THREADS, smem, st, p, tw);
-  return check_launch("clifford_log_prob_kernel");
+  return launch_persistent_pdl(clifford_log_prob_kernel<LOG2N, ROWK, FWD_ONLY, VM>, "clifford_log_prob_kernel", Pl::THREADS,
+                               smem, (p.rows + Pl::GROUPS - 1) / Pl::GROUPS, nullptr, st, p, tw);
 }
 
 template <bool ROWK, bool VM = false>
 int dispatch_lp(const CliffordLogProbParams& p, cudaStream_t st) {
-  const bool fast = is_pow2(p.d) && p.d >= 16 && p.d <= 8192 && aligned(p.value, 8);
-  if (fast) {
-    switch (ilog2(p.d)) {
-#define CVB_CASE(L) case L: return launch_lp_fast<L, ROWK, false, VM>(p, st);
-      CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-      CVB_CASE(13)
-#undef CVB_CASE
-    }
-  }
-  static const bool no_small = getenv("CVB_NO_SMALL_ROWS") != nullptr;
-  if (2 * p.d <= kSmallMaxN && !no_small) {
-    const int rt = small_rows_per_tile(p.rows, sm_count(), [&](int r) { return clifford_lp_small_smem(p.d, r); });
-    const size_t smem_s = clifford_lp_small_smem(p.d, rt);
-    auto kern_s = clifford_lp_small_kernel<ROWK, VM>;
-    int grid_s = 0;
-    if (int rc = persistent_grid(kern_s, kSmallThreads, smem_s, (p.rows + rt - 1) / rt, &grid_s)) return rc;
-    kern_s<<<grid_s, kSmallThreads, smem_s, st>>>(p, rt);
-    return check_launch("clifford_log_prob_small_kernel");
-  }
   const int n = 2 * p.d;
-  const size_t smem = sizeof(cplx) * n + sizeof(float) * (n + 32);
-  CVB_REQUIRE(smem <= kGenericSmemLimit, kUnsupported, "clifford log_prob: d=%d too large for the direct-DFT path", p.d);
-  auto kern = clifford_log_prob_generic_kernel<ROWK, VM>;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, kGenericThreads, smem, p.rows, &grid)) return rc;
-  kern<<<grid, kGenericThreads, smem, st>>>(p);
-  return check_launch("clifford_log_prob_generic_kernel");
+  return dispatch_clifford(
+      "clifford log_prob", p, n, p.value, [&](auto L) { return launch_lp_fast<decltype(L)::value, ROWK, false, VM>(p, st); },
+      clifford_lp_small_kernel<ROWK, VM>, [&](int r) { return clifford_lp_small_smem(p.d, r); },
+      clifford_log_prob_generic_kernel<ROWK, VM>, sizeof(cplx) * n + sizeof(float) * (n + 32), st);
 }
 
 }  // namespace

@@ -18,22 +18,22 @@ namespace {
 template <int FAMILY>
 int launch_sphere_rsample(const SphereParams& p, cudaStream_t st, const char* what) {
   const int grid = row_warp_grid(p.rows);
-  switch ((p.D + 127) / 128) {
-#define CVB_CASE(KK) case KK: sphere_rsample_reg_kernel<FAMILY, KK><<<grid, 256, 0, st>>>(p); break;
-    CVB_CASE(1) CVB_CASE(2) CVB_CASE(3) CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8)
-#undef CVB_CASE
-    default: sphere_rsample_kernel<FAMILY><<<grid, 256, 0, st>>>(p);
+  const int k = (p.D + 127) / 128;
+  if (k <= 8) {
+    with_int<1, 8>(k, [&](auto K) { sphere_rsample_reg_kernel<FAMILY, decltype(K)::value><<<grid, 256, 0, st>>>(p); return kOk; });
+  } else {
+    sphere_rsample_kernel<FAMILY><<<grid, 256, 0, st>>>(p);
   }
   return check_launch(what);
 }
 template <int FAMILY>
 int launch_sphere_rsample_bwd(const SphereParams& p, cudaStream_t st, const char* what) {
   const int grid = row_warp_grid(p.rows);
-  switch ((p.D + 127) / 128) {
-#define CVB_CASE(KK) case KK: sphere_rsample_bwd_reg_kernel<FAMILY, KK><<<grid, 256, 0, st>>>(p); break;
-    CVB_CASE(1) CVB_CASE(2) CVB_CASE(3) CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8)
-#undef CVB_CASE
-    default: sphere_rsample_bwd_kernel<FAMILY><<<grid, 256, 0, st>>>(p);
+  const int k = (p.D + 127) / 128;
+  if (k <= 8) {
+    with_int<1, 8>(k, [&](auto K) { sphere_rsample_bwd_reg_kernel<FAMILY, decltype(K)::value><<<grid, 256, 0, st>>>(p); return kOk; });
+  } else {
+    sphere_rsample_bwd_kernel<FAMILY><<<grid, 256, 0, st>>>(p);
   }
   return check_launch(what);
 }

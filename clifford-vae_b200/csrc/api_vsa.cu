@@ -1,5 +1,4 @@
 // C ABI entry points for the VSA / HRR kernels (include/clifford_b200.h).
-#include <cstdlib>
 #include "launch.cuh"
 #include "vsa_kernels.cuh"
 #include "../../include/clifford_b200.h"
@@ -12,19 +11,6 @@ extern "C" int cvb_internal_unitary(float* out, long long n, int d, float eps, u
                                     unsigned long long offset, void* stream);
 
 namespace {
-
-template <int LOG2N>
-int launch_depth_chain(const float* vecs, float* out, long long trials, int mp1, cudaStream_t st) {
-  using Pl = FftPlan<LOG2N>;
-  const cplx* tw = device_twiddles();
-  if (!tw) return kCudaError;
-  const size_t smem = sizeof(cplx) * Pl::XCH * Pl::GROUPS + sizeof(float) * 32 * Pl::GROUPS;
-  auto kern = depth_chain_kernel<LOG2N>;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, (trials + Pl::GROUPS - 1) / Pl::GROUPS, &grid)) return rc;
-  kern<<<grid, Pl::THREADS, smem, st>>>(vecs, out, trials, mp1, tw);
-  return check_launch("depth_chain_kernel");
-}
 
 __global__ void normal_fill_kernel(float* out, long long total, float scale, PhiloxKey key) {
   // each Philox call yields 4 normals
@@ -65,14 +51,14 @@ int cvb_vsa_depth_chain_cosine(const float* vecs, float* out, long long trials, 
   CVB_REQUIRE(vecs && out && trials > 0 && m_plus_1 >= 1, kBadArgument, "cvb_vsa_depth_chain_cosine: bad arguments");
   CVB_REQUIRE(is_pow2(d) && d >= 32 && d <= 16384 && aligned(vecs, 8), kUnsupported,
               "cvb_vsa_depth_chain_cosine: d=%d must be a power of two in [32, 16384] (use bind/unbind otherwise)", d);
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (ilog2(d) - 1) {
-#define CVB_CASE(L) case L: return launch_depth_chain<L>(vecs, out, trials, m_plus_1, st);
-    CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-    CVB_CASE(13)
-#undef CVB_CASE
-  }
-  return kUnsupported;
+  return with_int<4, 13>(ilog2(d) - 1, [&](auto L) -> int {
+    using Pl = FftPlan<decltype(L)::value>;
+    const cplx* tw = device_twiddles();
+    if (!tw) return kCudaError;
+    return launch_persistent(depth_chain_kernel<decltype(L)::value>, "depth_chain_kernel", Pl::THREADS,
+                             sizeof(cplx) * Pl::XCH * Pl::GROUPS + sizeof(float) * 32 * Pl::GROUPS,
+                             (trials + Pl::GROUPS - 1) / Pl::GROUPS, (cudaStream_t)stream, vecs, out, trials, m_plus_1, tw);
+  });
 }
 
 int cvb_vsa_invert(const float* a, float* out, long long rows, int d, void* stream) {

@@ -1,7 +1,6 @@
 // Launch helpers for the bind family, shared by the api_vsa_bind_*.cu translation units (the 10 sizes x 5 modes
 // are split over two units to keep the build parallel).
 #pragma once
-#include <cstdlib>
 #include "launch.cuh"
 #include "vsa_kernels.cuh"
 
@@ -13,94 +12,48 @@ int launch_bind_fast(const BindParams& p_in, cudaStream_t st) {
   using Pl = WideFftPlan<LOG2N>;
   const cplx* tw = device_twiddles();
   if (!tw) return kCudaError;
-  // CVB_BIND_VARIANT (experiments): "staged" (TMA-staged rows) or "direct" (plain loads); default by size
-  static const char* variant = getenv("CVB_BIND_VARIANT");
   const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  int grid = 0;
-  static const bool static_sched = getenv("CVB_STATIC_SCHEDULE") != nullptr;
-  // staging mode measured on B200 (tools/bench_ops.py): 0 = plain loads, 2 = a and b through TMA (1 = a only was measured too: no gain)
-  int mode = (LOG2N >= 12) ? 2 : 0;
-  if (variant) mode = (variant[0] == 's') ? 2 : 0;
-  if (!(aligned(p.a, 16) && aligned(p.b, 16))) mode = 0;
-  if constexpr (LOG2N < 11) mode = 0;      // small rows: plain loads always won; skip instantiating the staged variant
-  if (mode == 2) {
-    const size_t smem = bind_v3_smem_bytes<LOG2N, 2>();
-    if constexpr (LOG2N >= 11) {
-      auto kern = bind_v3_kernel<LOG2N, MODE, 2>;
-      if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
-      p.sched = (!static_sched && work > grid) ? next_sched_slot() : nullptr;
-    launch_pdl(kern, grid, Pl::THREADS, smem, st, p, tw);
-      return check_launch("bind_v3_kernel<staged ab>");
-    }
+  // staging measured on B200 (tools/bench_ops.py, DESIGN.md section 4): a and b through TMA from d = 8192 up (a only was
+  // measured too: no gain); shorter rows use plain loads, and the staged variant is not instantiated for them
+  if constexpr (LOG2N >= 12) {
+    if (aligned(p.a, 16) && aligned(p.b, 16))
+      return launch_persistent_pdl(bind_v3_kernel<LOG2N, MODE, 2>, "bind_v3_kernel<staged ab>", Pl::THREADS,
+                                   bind_v3_smem_bytes<LOG2N, 2>(), work, &p.sched, st, p, tw);
   }
-  const size_t smem = bind_v3_smem_bytes<LOG2N, 0>();
-  auto kern = bind_v3_kernel<LOG2N, MODE, 0>;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
-  p.sched = (!static_sched && work > grid) ? next_sched_slot() : nullptr;
-  launch_pdl(kern, grid, Pl::THREADS, smem, st, p, tw);
-  return check_launch("bind_v3_kernel<direct>");
-}
-
-template <int LOG2N, int MODE>
-int launch_bind_pad(const BindParams& p, int d, cudaStream_t st) {
-  using Pl = WideFftPlan<LOG2N>;
-  const cplx* tw = device_twiddles();
-  if (!tw) return kCudaError;
-  const size_t smem = bind_pad_smem_bytes<LOG2N>();
-  auto kern = bind_pad_kernel<LOG2N, MODE>;
-  const long long work = (p.rows + Pl::GROUPS - 1) / Pl::GROUPS;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, Pl::THREADS, smem, work, &grid)) return rc;
-  kern<<<grid, Pl::THREADS, smem, st>>>(p, d, tw);
-  return check_launch("bind_pad_kernel");
+  return launch_persistent_pdl(bind_v3_kernel<LOG2N, MODE, 0>, "bind_v3_kernel<direct>", Pl::THREADS,
+                               bind_v3_smem_bytes<LOG2N, 0>(), work, &p.sched, st, p, tw);
 }
 
 template <int MODE>
 int dispatch_bind(const BindParams& p, int d, cudaStream_t st) {
   const bool fast = is_pow2(d) && d >= 32 && d <= 16384 && aligned(p.a, 8) && aligned(p.b, 8) && aligned(p.out, 8);
-  if (fast) {
-    switch (ilog2(d) - 1) {
-#define CVB_CASE(L) case L: return launch_bind_fast<L, MODE>(p, st);
-      CVB_CASE(4) CVB_CASE(5) CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12)
-      CVB_CASE(13)
-#undef CVB_CASE
-    }
-  }
+  if (fast) return with_int<4, 13>(ilog2(d) - 1, [&](auto L) { return launch_bind_fast<decltype(L)::value, MODE>(p, st); });
   // any other length: the bilinear modes fold a zero-padded power-of-two convolution (bind_pad_kernel) once the
   // O(d^2) direct DFT would cost more (d > 48); the quotient modes need the true length-d spectrum (direct DFT)
-  static const bool no_pad = getenv("CVB_BIND_NO_PAD") != nullptr;      // A/B switch for tools/bench_small_dims.py
-  static const bool no_small = getenv("CVB_NO_SMALL_ROWS") != nullptr;  // A/B switch: one CTA per pair at short lengths
   constexpr bool kBilinear = (MODE == kBindMul || MODE == kBindMulConj || MODE == kBindNegMulConj);
-  if (d <= kBindSmallMaxD && !no_small && (!kBilinear || d <= 48 || no_pad)) {
+  if (d <= kBindSmallMaxD && (!kBilinear || d <= 48)) {
     // short vectors: a tile of pairs per CTA (rows per tile sized so that small batches stay spread over the SMs)
     int rt = 32;
     while (rt > 4 && ((p.rows + rt - 1) / rt < 2LL * sm_count() || bind_small_smem(d, rt) > 48 * 1024)) rt >>= 1;
-    const size_t smem_s = bind_small_smem(d, rt);
-    auto kern_s = bind_small_kernel<MODE>;
-    int grid_s = 0;
-    if (int rc = persistent_grid(kern_s, kBindSmallThreads, smem_s, (p.rows + rt - 1) / rt, &grid_s)) return rc;
-    kern_s<<<grid_s, kBindSmallThreads, smem_s, st>>>(p, d, rt);
-    return check_launch("bind_small_kernel");
+    return launch_persistent(bind_small_kernel<MODE>, "bind_small_kernel", kBindSmallThreads, bind_small_smem(d, rt),
+                             (p.rows + rt - 1) / rt, st, p, d, rt);
   }
-  if constexpr (MODE == kBindMul || MODE == kBindMulConj || MODE == kBindNegMulConj) {
-    if (d > 48 && d <= 8192 && !no_pad) {
+  if constexpr (kBilinear) {
+    if (d > 48 && d <= 8192) {
       int log2m = 1;
       while ((1 << log2m) < 2 * d) ++log2m;
-      switch (log2m - 1) {
-#define CVB_CASE(L) case L: return launch_bind_pad<L, MODE>(p, d, st);
-        CVB_CASE(6) CVB_CASE(7) CVB_CASE(8) CVB_CASE(9) CVB_CASE(10) CVB_CASE(11) CVB_CASE(12) CVB_CASE(13)
-#undef CVB_CASE
-      }
+      return with_int<6, 13>(log2m - 1, [&](auto L) -> int {
+        using Pl = WideFftPlan<decltype(L)::value>;
+        const cplx* tw = device_twiddles();
+        if (!tw) return kCudaError;
+        return launch_persistent(bind_pad_kernel<decltype(L)::value, MODE>, "bind_pad_kernel", Pl::THREADS,
+                                 bind_pad_smem_bytes<decltype(L)::value>(), (p.rows + Pl::GROUPS - 1) / Pl::GROUPS, st, p, d, tw);
+      });
     }
   }
   const size_t smem = sizeof(cplx) * d + sizeof(float) * (2 * d + 2) + sizeof(cplx) * (d / 2 + 1);
-  CVB_REQUIRE(smem <= 200 * 1024, kUnsupported, "vsa bind: d=%d too large for the direct-DFT path", d);
-  auto kern = bind_generic_kernel<MODE>;
-  int grid = 0;
-  if (int rc = persistent_grid(kern, 256, smem, p.rows, &grid)) return rc;
-  kern<<<grid, 256, smem, st>>>(p, d);
-  return check_launch("bind_generic_kernel");
+  CVB_REQUIRE(smem <= kGenericSmemLimit, kUnsupported, "vsa bind: d=%d too large for the direct-DFT path", d);
+  return launch_persistent(bind_generic_kernel<MODE>, "bind_generic_kernel", 256, smem, p.rows, st, p, d);
 }
-
 
 }  // namespace cvb

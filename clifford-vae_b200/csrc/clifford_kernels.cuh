@@ -15,34 +15,23 @@
 #include "special.cuh"
 // Minimum resident CTAs per SM requested for the forward kernel's 128-thread configurations (register cap 102 at 5).
 // Measured on B200 (device RNG, >= 1 GiB per launch): 5 beats 4 by 2-4 % at d = 512 / 2048 and loses 2 % at d = 1024.
-#ifndef CVB_FWD_MINB
-#define CVB_FWD_MINB 5
-#endif
+constexpr int kFwdMinBlocks = 5;
 // backward: 5 resident CTAs help at d = 2048 (+7 %) and d = 512 (+6 %), hurt at d = 1024 (-2 %); log_prob: 4 is best at every size
 template <int LOG2N>
 constexpr int clifford_bwd_min_blocks() { return LOG2N == 10 ? 4 : 5; }
-#ifndef CVB_FWD_BIND_MINB
-#define CVB_FWD_BIND_MINB 4
-#endif
 // the fused-bind variant carries a second set of transforms; since its pair stage forms each (k, N-k) pair once it fits 124
 // registers without spilling: 4 resident CTAs / SM measured 0.1166 -> 0.1069 ms at the headline shape (3 before; 5 does not
 // fit the shared memory)
-#ifndef CVB_FWD_KEEP_OWN
-#define CVB_FWD_KEEP_OWN 1
-#endif
-#ifndef CVB_ICDF_LOOP_UNROLL
-#define CVB_ICDF_LOOP_UNROLL 4
-#endif
+constexpr int kFwdBindMinBlocks = 4;
 // The lean forward sampler at d = 2048: its shared memory (33.9 KB per CTA) admits 6 resident CTAs, so the register cap
 // is set for 6 (85 registers) -- room to keep a table row's own phasors in registers between the sampling loop and the
-// C2R pre-tangle (CVB_FWD_KEEP_OWN: -16 shared-memory reads per thread and row, +3 %; at the 72-register cap of 7 CTAs
+// C2R pre-tangle (kFwdKeepOwn: -16 shared-memory reads per thread and row, +3 %; at the 72-register cap of 7 CTAs
 // that spills 116 bytes and loses 10 %).
-#ifndef CVB_FWD_LEAN_MINB
-#define CVB_FWD_LEAN_MINB 6
-#endif
+constexpr int kFwdLeanMinBlocks = 6;
+constexpr bool kFwdKeepOwn = true;
 template <int LOG2N, bool BIND = false, bool LEAN = false>
 constexpr int clifford_fwd_min_blocks() {
-  return BIND ? CVB_FWD_BIND_MINB : ((LEAN && LOG2N == 11) ? CVB_FWD_LEAN_MINB : (LOG2N == 10 ? 4 : CVB_FWD_MINB));
+  return BIND ? kFwdBindMinBlocks : ((LEAN && LOG2N == 11) ? kFwdLeanMinBlocks : (LOG2N == 10 ? 4 : kFwdMinBlocks));
 }
 
 namespace cvb {
@@ -98,16 +87,13 @@ __device__ __forceinline__ float fwd_row_kappa(const CliffordFwdParams& p, long 
 constexpr float kEps = 1e-7f;
 // the forward sampler's table carries the padding cell of icdf_build_row<.., PAD> (index = floor(x) unclamped)
 constexpr int kFwdIcdfCells = kIcdfCells + 1;
-constexpr int kIcdfLoopUnroll = CVB_ICDF_LOOP_UNROLL;   // Philox calls (4 circles each) of the table sampling loop unrolled together
+constexpr int kIcdfLoopUnroll = 4;   // Philox calls (4 circles each) of the table sampling loop unrolled together
 // the reference's atan2(s sqrt(max(1 - t^2, eps)), t) (clifford.py:44-48) never returns a phase below sqrt(eps) or above
 // pi - sqrt(eps): the table sampler clamps |phi| to that range
 constexpr float kIcdfPhiMin = 3.16227766e-4f, kIcdfPhiMax = 3.14127642f;
-#ifndef CVB_TABLE_COORD_MIN_LOG2N
-#define CVB_TABLE_COORD_MIN_LOG2N 9
-#endif
 // which row lengths save the table coordinate instead of t' on table-sampled rows (see clifford_bwd_smem_bytes)
 template <int LOG2N>
-constexpr bool clifford_saves_table_coord() { return LOG2N >= CVB_TABLE_COORD_MIN_LOG2N; }
+constexpr bool clifford_saves_table_coord() { return LOG2N >= 9; }
 
 __device__ __forceinline__ float sign_from_normal(float g) { return g / (fabsf(g) + kEps); }
 
@@ -575,7 +561,7 @@ clifford_fwd_kernel(const CliffordFwdParams p, const cplx* __restrict__ tw, cons
     };
     // phase 1: phasors of the half spectrum into the exchange buffer (lightly unrolled: small code, some ILP)
     const bool table_row = ICDF && icdf_row_ok(kap_row);      // uniform over the group
-    constexpr bool KEEP_OWN = CVB_FWD_KEEP_OWN && ICDF && !BIND;    // table rows keep their own phasors in registers
+    constexpr bool KEEP_OWN = kFwdKeepOwn && ICDF && !BIND;    // table rows keep their own phasors in registers
     cplx xown[KEEP_OWN ? E : 1];
     if (ICDF && table_row) {
       // device RNG through the row's inverse-CDF cells: one Philox call per FOUR circles, no rejection, no queue

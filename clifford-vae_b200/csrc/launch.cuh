@@ -1,8 +1,8 @@
 // Host-side launch plumbing shared by the api_*.cu translation units.
 #pragma once
-#include <cstdlib>
 #include <cstdio>
 #include <atomic>
+#include <type_traits>
 #include "common.cuh"
 #include "rng.cuh"
 
@@ -65,8 +65,6 @@ inline int persistent_grid(Kernel kernel, int threads, size_t smem, long long wo
     set_last_error("kernel does not fit on an SM (threads=%d smem=%zu)", threads, smem);
     return kUnsupported;
   }
-  static const int cap = getenv("CVB_MAX_CTAS_PER_SM") ? atoi(getenv("CVB_MAX_CTAS_PER_SM")) : 0;   // tuning knob
-  if (cap > 0 && per_sm > cap) per_sm = cap;
   long long g = (long long)sm_count() * per_sm;
   if (g > work_ctas) g = work_ctas;
   if (g < 1) g = 1;
@@ -91,13 +89,29 @@ inline PhiloxKey make_key(unsigned long long seed, unsigned long long offset, ui
   return k;
 }
 
-// Programmatic dependent launch (sm_90+): the kernel is allowed to become resident while its predecessor on the stream
-// drains; it blocks at pdl_wait() (griddepcontrol.wait) -- its first statement, before any global access to caller data --
-// until the predecessor has completed and flushed.  That removes the launch / scheduling gap between the back-to-back
-// kernels of a step (sampler -> bind -> sampler ...).  CVB_NO_PDL=1 restores plain launches (A/B switch).
+// Persistent launch: persistent_grid -> launch -> check_launch.  `args` are the kernel's arguments.
+template <typename Kernel, typename... Args>
+inline int launch_persistent(Kernel kern, const char* what, int threads, size_t smem, long long work, cudaStream_t st,
+                             const Args&... args) {
+  int grid = 0;
+  if (int rc = persistent_grid(kern, threads, smem, work, &grid)) return rc;
+  kern<<<grid, threads, smem, st>>>(args...);
+  return check_launch(what);
+}
+
+// The same with programmatic dependent launch (sm_90+): the kernel is allowed to become resident while its predecessor
+// on the stream drains; it blocks at pdl_wait_and_release() (griddepcontrol.wait) -- its first statement, before any
+// global access to caller data -- until the predecessor has completed and flushed.  That removes the launch / scheduling
+// gap between the back-to-back kernels of a step (sampler -> bind -> sampler ...).  Only for kernels that begin with
+// pdl_wait_and_release(): one without the wait would read its inputs before the predecessor has written them.
+// `sched` (or null): the schedule word of the params among `args`, which are passed on only after it is set -- a
+// dynamic-schedule slot when the CTAs loop over rows (work > grid), else null.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), int grid, int threads, size_t smem, cudaStream_t st, Args... args) {
-  static const bool no_pdl = getenv("CVB_NO_PDL") != nullptr;
+inline int launch_persistent_pdl(void (*kern)(KArgs...), const char* what, int threads, size_t smem, long long work,
+                                 int** sched, cudaStream_t st, const Args&... args) {
+  int grid = 0;
+  if (int rc = persistent_grid(kern, threads, smem, work, &grid)) return rc;
+  if (sched) *sched = work > grid ? next_sched_slot() : nullptr;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3((unsigned)threads);
@@ -107,9 +121,25 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), int grid, int threads, siz
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = no_pdl ? 0 : 1;
-  return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
+  cfg.numAttrs = 1;
+  cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
+  return check_launch(what);
 }
+
+// Calls f(std::integral_constant<int, V>{}) for the run-time value v in [LO, HI] and returns its result; returns
+// `otherwise` for any other v.  Fans a run-time size out to the kernel instantiation for it.
+template <int LO, int HI, typename F>
+inline int with_int(int v, F&& f, int otherwise = kUnsupported) {
+  if constexpr (LO <= HI) {
+    if (v == LO) return f(std::integral_constant<int, LO>{});
+    return with_int<LO + 1, HI>(v, f, otherwise);
+  } else {
+    return otherwise;
+  }
+}
+
+// The direct-DFT kernels (Clifford and bind) keep a row's transform in shared memory: longer rows are refused.
+constexpr size_t kGenericSmemLimit = 200 * 1024;
 
 inline bool is_pow2(long long x) { return x > 0 && (x & (x - 1)) == 0; }
 inline int ilog2(long long x) { int l = 0; while ((1LL << l) < x) ++l; return l; }

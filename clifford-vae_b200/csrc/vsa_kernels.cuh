@@ -4,9 +4,6 @@
 #pragma once
 #include "fft_core.cuh"
 #include "tma.cuh"
-#ifndef CVB_BIND_MINB
-#define CVB_BIND_MINB 4
-#endif
 
 namespace cvb {
 
@@ -91,8 +88,10 @@ __device__ __forceinline__ void bind_pair(const cplx* park, const cplx* xch, con
   vkp = cconj(cscale(csub(s, d), fold));
 }
 
+// resident CTAs per SM requested for the 128-thread plans of 16 points per thread
+constexpr int kBindMinBlocks = 4;
 template <int LOG2N, int MODE, int STAGED>
-__global__ void __launch_bounds__(WideFftPlan<LOG2N>::THREADS, (WideFftPlan<LOG2N>::THREADS <= 128 ? (WideFftPlan<LOG2N>::E > 16 ? 2 : CVB_BIND_MINB) : ((WideFftPlan<LOG2N>::THREADS <= 256 && WideFftPlan<LOG2N>::E <= 16) ? 2 : 1)))
+__global__ void __launch_bounds__(WideFftPlan<LOG2N>::THREADS, (WideFftPlan<LOG2N>::THREADS <= 128 ? (WideFftPlan<LOG2N>::E > 16 ? 2 : kBindMinBlocks) : ((WideFftPlan<LOG2N>::THREADS <= 256 && WideFftPlan<LOG2N>::E <= 16) ? 2 : 1)))
 bind_v3_kernel(const BindParams p, const cplx* __restrict__ tw) {
   pdl_wait_and_release();
   using Pl = WideFftPlan<LOG2N>;

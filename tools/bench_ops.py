@@ -32,7 +32,7 @@ if what in ("bind", "all"):
         a = torch.randn(N, dd, device=dev); b = torch.randn(N, dd, device=dev); o = torch.empty(N, dd, device=dev)
         ms = timeit(lambda: lib.cvb_vsa_bind(a.data_ptr(), b.data_ptr(), o.data_ptr(), N, N, N, dd, 0, st))
         gb = N * 12 * dd / (ms * 1e-3) / 1e9
-        print(f"bind d={dd:6d} N={N:7d} {ms:8.3f} ms {N/(ms*1e-3):.3e} vec/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}% [{os.environ.get('CVB_BIND_VARIANT','default')}]")
+        print(f"bind d={dd:6d} N={N:7d} {ms:8.3f} ms {N/(ms*1e-3):.3e} vec/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}%")
         del a, b, o
 if what in ("clifford", "all"):
     for B, d in ((4096, 2048), (65536, 2048), (262144, 512), (131072, 1024)):

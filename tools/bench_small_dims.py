@@ -1,6 +1,5 @@
 """Timing of the small and non-power-of-two lengths the reference's drivers use (SURVEY.md 8(f) item 4):
-python tools/bench_small_dims.py   (run it twice for the A/B of the padded-FFT bind: CVB_BIND_NO_PAD=1 forces the
-O(d^2) direct-DFT kernel for every non-power-of-two length)."""
+python tools/bench_small_dims.py"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "clifford-vae_b200")]
@@ -20,8 +19,6 @@ class _Checked:
 
 lib = _Checked()
 PEAK = 6548.8
-tag = "direct-DFT only" if os.environ.get("CVB_BIND_NO_PAD") else "default"
-small = "one CTA per row" if os.environ.get("CVB_NO_SMALL_ROWS") else "row tiles"
 
 
 def timeit(fn, reps=10):
@@ -46,7 +43,7 @@ for d in (2, 5, 10, 20, 40, 64, 100, 200, 300):
     loc = torch.randn(B, d, device=dev); kap = torch.rand(B, device=dev) * 9 + 0.1; z = torch.empty(B, 2 * d, device=dev); kl = torch.empty(B, device=dev)
     ms = timeit(lambda: lib.cvb_clifford_ps_rsample(loc.data_ptr(), kap.data_ptr(), 1, 0, B, None, None, 7, 0, z.data_ptr(), None, None, kl.data_ptr(), None, B, d, st))
     gb = B * (12 * d + 8) / ms / 1e6
-    print(f"clifford fwd rng      d={d:5d} B={B:8d} {ms:8.3f} ms {B/ms*1e3:.3e} rows/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}%  (direct DFT, n={2*d}, {small if 2 * d <= 512 else "one CTA per row"})")
+    print(f"clifford fwd rng      d={d:5d} B={B:8d} {ms:8.3f} ms {B/ms*1e3:.3e} rows/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}%  (direct DFT, n={2*d}, {"row tiles" if 2 * d <= 512 else "one CTA per row"})")
     if d <= 256:
         # backward and log_prob of the same rows
         gz = torch.randn(B, 2 * d, device=dev); tps = torch.rand(B, d, device=dev) * 0.98 + 0.01; dl = torch.empty(B, d, device=dev); dk = torch.empty(B, device=dev)
@@ -74,5 +71,5 @@ for d in (4, 10, 21, 41, 80, 100, 129, 144, 484, 513, 1000, 3000):
     for name, mode in (("bind", 0), ("unbind inv", 1), ("unbind deconv", 2)):
         ms = timeit(lambda: lib.cvb_vsa_bind(a.data_ptr(), b.data_ptr(), o.data_ptr(), N, N, N, d, mode, st), reps=5)
         gb = N * 12 * d / ms / 1e6
-        print(f"{name:14s} [{tag}] d={d:5d} N={N:8d} {ms:8.3f} ms {N/ms*1e3:.3e} vec/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}%")
+        print(f"{name:14s} d={d:5d} N={N:8d} {ms:8.3f} ms {N/ms*1e3:.3e} vec/s {gb:7.1f} GB/s {100*gb/PEAK:5.1f}%")
     del a, b, o

@@ -11,7 +11,6 @@ python bench.py > $O/r2f_bench.json 2> $O/r2f_bench.err
 python bench.py --impl reference > $O/r2f_ref.json 2> $O/r2f_ref.err
 python tools/bench_ops.py all > $O/r2f_bench_ops.txt 2>&1
 python tools/bench_small_dims.py > $O/r2f_small_dims.txt 2>&1
-CVB_NO_SMALL_ROWS=1 python tools/bench_small_dims.py 2>&1 | grep -v "d=  1[0-9][0-9] \|d=  [2-9][0-9][0-9]\|d= [0-9][0-9][0-9][0-9]" > $O/r2f_small_dims_one_cta_per_row.txt
 python tools/bench_latency.py > $O/r2f_latency.txt 2>&1
 python tools/bench_prologue.py > $O/r2f_prologue.txt 2>&1
 BENCH="python bench.py --steps 3 --warmup 3 --no-cpu-baseline --no-vae-step --no-other-configs"

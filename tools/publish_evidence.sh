@@ -13,7 +13,6 @@ cp $O/r2f_ncu_summary_bench.txt profiles/r02_ncu_summary_bench_fwd_bind.txt
 cp $O/r2f_ncu_summary_bwd_lp.txt profiles/r02_ncu_bwd_logprob_v2.txt
 cp $O/r2f_ncu_summary_small.txt profiles/r02_ncu_summary_small_rows.txt
 cp $O/r2f_small_dims.txt profiles/r02_small_dims.txt
-cp $O/r2f_small_dims_one_cta_per_row.txt profiles/r02_small_dims_one_cta_per_row.txt
 cp $O/r2f_latency.txt profiles/r02_latency.txt
 cp $O/r2f_prologue.txt profiles/r02_sampler_prologue.txt
 cp $O/r2f_bench_ops.txt profiles/r02_bench_ops.txt
