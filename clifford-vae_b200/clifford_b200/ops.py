@@ -148,6 +148,11 @@ class CliffordPSRsample(torch.autograd.Function):
         dloc = dkap = None
         if grad_z is not None:
             gz = _f32c(grad_z)
+            if gz.data_ptr() % 16:
+                # a contiguous view at an odd offset (e.g. the gradient of torch.cat([s.view(1), z.flatten()])): the FFT
+                # engine needs 8-byte aligned gradient rows, and at power-of-two d >= 512 the saved device draws can only
+                # be read there (the library refuses the call otherwise)
+                gz = gz.clone()
             dloc_rows = torch.empty(rows, d, device=gz.device, dtype=torch.float32)
             dk_rows = torch.empty((rows,) if kes == 0 else (rows, d), device=gz.device, dtype=torch.float32)
             if ctx.head is None:

@@ -45,6 +45,10 @@ static int clifford_ps_rsample_backward_impl(const float* grad_z, const float* l
   CVB_REQUIRE(grad_z && loc && kappa && dloc && dkappa, kBadArgument, "cvb_clifford_ps_rsample_backward: null pointer");
   CVB_REQUIRE(rows > 0 && d >= 1 && loc_rows > 0, kBadArgument, "cvb_clifford_ps_rsample_backward: bad sizes");
   CVB_REQUIRE(tp_signed || (tprime && gnoise), kBadArgument, "cvb_clifford_ps_rsample_backward: need tp_signed or (tprime, gnoise)");
+  // every tier reads tp_signed whenever it is given, injected draws or not
+  CVB_REQUIRE(!tp_signed || !ps_saved_draws_need_fft(d, kappa_el_stride == 0) || aligned(grad_z, 8), kUnsupported,
+              "cvb_clifford_ps_rsample_backward: grad_z must be 8-byte aligned with tp_signed at d=%d and one concentration "
+              "per row (the forward saved those draws in the FFT engine's format)", d);
   CliffordBwdParams p{};
   p.grad_z = grad_z; p.loc = loc; p.kappa = kappa; p.kappa_row_stride = kappa_row_stride;
   p.kappa_el_stride = kappa_el_stride; p.loc_rows = (int)loc_rows; p.tprime = tprime; p.gnoise = gnoise;

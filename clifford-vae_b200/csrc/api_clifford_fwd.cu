@@ -66,6 +66,9 @@ static int clifford_ps_rsample_impl(const float* loc, const float* kappa, long l
   CVB_REQUIRE((tprime == nullptr) == (gnoise == nullptr), kBadArgument, "cvb_clifford_ps_rsample: give both tprime and gnoise or neither");
   CVB_REQUIRE(kappa_el_stride == 0 || (!entropy && !kl && !dentropy), kBadArgument,
               "cvb_clifford_ps_rsample: fused entropy/kl needs one concentration per row; use cvb_ps_entropy_kl");
+  CVB_REQUIRE(tprime || !tp_signed || !ps_saved_draws_need_fft(d, kappa_el_stride == 0) || aligned(z, 8), kUnsupported,
+              "cvb_clifford_ps_rsample: z must be 8-byte aligned to save tp_signed in RNG mode at d=%d with one "
+              "concentration per row (the backward reads those draws in the FFT engine's format)", d);
   CliffordFwdParams p{};
   p.loc = loc; p.kappa = kappa; p.kappa_row_stride = kappa_row_stride; p.kappa_el_stride = kappa_el_stride;
   p.loc_rows = (int)loc_rows; p.tprime = tprime; p.gnoise = gnoise; p.z = z; p.tp_signed = tp_signed;

@@ -24,4 +24,12 @@ int dispatch_clifford(const char* what, const P& p, int n, const void* out, Fft 
   return launch_persistent(generic, what, kGenericThreads, generic_smem, p.rows, st, p);
 }
 
+// Whether the power-spherical draws a device-RNG forward saves for its backward (tp_signed) depend on the kernel tier.
+// With one concentration per row and a power-of-two d in [512, 8192] the FFT engine saves the signed table coordinate
+// of table-sampled rows (clifford_saves_table_coord); the row-tile and direct-DFT kernels save and read copysign(t', s).
+// dispatch_clifford picks the tier from the alignment of z (forward) and grad_z (backward), so at these lengths both
+// must be 8-byte aligned: otherwise one of the two calls would read the other's format as its own.
+static_assert(clifford_saves_table_coord<9>() && !clifford_saves_table_coord<8>(), "table coordinates from d = 512 up");
+inline bool ps_saved_draws_need_fft(int d, bool rowk) { return rowk && is_pow2(d) && d >= 512 && d <= 8192; }
+
 }  // namespace cvb

@@ -55,7 +55,9 @@ CVB_API long long cvb_launch_count(void);
  * with Philox4x32-10 keyed by (seed, offset).  Outputs: z (rows, 2d); optional tp_signed (rows, d):
  * the draws saved for cvb_clifford_ps_rsample_backward in RNG mode -- OPAQUE to the caller: copysign(t', sign), or, on
  * rows sampled through the inverse-CDF table (one concentration <= 32 per row, power-of-two d >= 512), the signed table
- * coordinate of the draw; element 0 of every row is left unwritten; optional entropy / kl / dentropy (rows)
+ * coordinate of the draw; element 0 of every row is left unwritten.  With one concentration per row and a power-of-two
+ * d in [512, 8192], saving tp_signed in RNG mode needs z 8-byte aligned (else CVB_UNSUPPORTED): the saved format
+ * depends on the kernel, and the kernel on z's alignment; optional entropy / kl / dentropy (rows)
  * (dentropy = d entropy / d kappa), written only when kappa_el_stride == 0 (otherwise call
  * cvb_ps_entropy_kl). */
 CVB_API int cvb_clifford_ps_rsample(const float* loc, const float* kappa, long long kappa_row_stride, int kappa_el_stride,
@@ -67,7 +69,9 @@ CVB_API int cvb_clifford_ps_rsample(const float* loc, const float* kappa, long l
  * Give either (tprime, gnoise) [injected draws: ATen's piecewise implicit Beta gradient, like the reference] or the
  * tp_signed buffer the forward wrote for the SAME (loc, kappa, rows, d) [table-sampled rows: the pathwise derivative of the
  * table map itself, i.e. the same implicit reparameterisation gradient evaluated to 2.5e-5 instead of ATen's
- * approximation of it].  dloc (rows, d); dkappa (rows) when kappa_el_stride == 0, else (rows, d). */
+ * approximation of it].  With tp_signed, one concentration per row and a power-of-two d in [512, 8192], grad_z must be
+ * 8-byte aligned (else CVB_UNSUPPORTED), like the forward's z.  dloc (rows, d); dkappa (rows) when kappa_el_stride == 0,
+ * else (rows, d). */
 CVB_API int cvb_clifford_ps_rsample_backward(const float* grad_z, const float* loc, const float* kappa,
                                      long long kappa_row_stride, int kappa_el_stride, long long loc_rows,
                                      const float* tprime, const float* gnoise, const float* tp_signed, float* dloc,

@@ -1,4 +1,6 @@
 """GPU parity: utils.vsa ops (ctypes -> C ABI) vs golden vectors from the reference and the oracle."""
+import math
+
 import numpy as np
 import pytest
 import torch
@@ -71,6 +73,24 @@ def test_bind_all_sizes_vs_oracle_and_identities(d):
     assert rel_err(vsa.unbind(ag, bg, "inv").cpu(), O.unbind(a, b, "inv")) < 1e-5
     # unbind == bind with the explicit invert
     assert rel_err(vsa.unbind(ag, bg, "inv").cpu(), vsa.bind(ag, vsa.invert(bg)).cpu()) < 1e-5
+    # the quotient modes (2: A / (B + 1e-12), 3: A / conj(B + 1e-12)) and the adjoint mode 4 (-A conj B) against float64,
+    # with a well-conditioned b (spectrum magnitudes in [0.5, 2], random phases) so that the quotients hold 1e-5 too
+    from clifford_b200 import _lib
+    h = d // 2 + 1
+    mag = 0.5 * 4.0 ** torch.rand(k, h, dtype=torch.float64)
+    Bh = torch.polar(mag, 2 * math.pi * torch.rand(k, h, dtype=torch.float64))
+    Bh[:, 0] = mag[:, 0]                               # the bins irfft keeps real
+    if d % 2 == 0:
+        Bh[:, -1] = mag[:, -1]
+    bq = torch.fft.irfft(Bh, n=d).float()
+    A, Bf = torch.fft.fft(a.double()), torch.fft.fft(bq.double())
+    want = {2: A / (Bf + 1e-12), 3: A / (Bf + 1e-12).conj(), 4: -A * Bf.conj()}
+    bqd = bq.to(DEV)
+    for mode, ref in want.items():
+        out = torch.empty(k, d, device=DEV)
+        _lib.check(_lib.load().cvb_vsa_bind(ag.data_ptr(), bqd.data_ptr(), out.data_ptr(), k, k, k, d, mode,
+                                            torch.cuda.current_stream().cuda_stream), f"bind mode {mode}")
+        assert rel_err(out.cpu(), torch.fft.ifft(ref).real) < 1e-5, mode
 
 
 @pytest.mark.parametrize("d", [64, 1024, 37])
