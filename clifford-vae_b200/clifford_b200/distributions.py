@@ -27,6 +27,21 @@ def head_concentration(raw_scale, floor, kmax):
     return torch.clamp(torch.nn.functional.softplus(raw_scale) + floor, max=kmax)
 
 
+def _stale(cached, param) -> bool:
+    """A row scalar cached by a no-grad or forward-only call carries no graph: it is recomputed when autograd now wants
+    its gradient with respect to `param` (the concentration, or the raw head output of a head-built distribution)."""
+    return ops._wants_graph(param) and not cached.requires_grad
+
+
+def _keep_fused(dist, name, param, shape, *pairs):
+    """Cache in dist.<name>, for entropy() / kl_divergence / log_prob, the row scalars that rsample's launch produced:
+    (value, d value / d param) pairs, each re-attached to `param` and shaped `shape`; one pair is cached as a tensor,
+    several as a tuple.  A launch that produced none (empty values) keeps the earlier cache."""
+    if pairs[0][0].numel():
+        vals = tuple(ops.row_scalar(param, v, dv).reshape(shape) for v, dv in pairs)
+        setattr(dist, name, vals[0] if len(vals) == 1 else vals)
+
+
 def _numel(shape) -> int:
     n = 1
     for s in shape:
@@ -127,8 +142,7 @@ class PowerSpherical(Distribution):
             loc2, kap = self._flat()
             param = self.scale
             z, ent, dent = ops.PowerSphericalRsample.apply(loc2, kap, n, _base_draws)
-        if ent.numel():                                             # same launch; entropy() / kl_divergence reuse it
-            self._fused_entropy = ops.row_scalar(param, ent, dent).reshape(param.shape)
+        _keep_fused(self, "_fused_entropy", param, param.shape, (ent, dent))
         return z.reshape(tuple(sample_shape) + tuple(self.batch_shape) + (self.dim,)).to(self.loc.dtype)
 
     def sample(self, sample_shape=torch.Size()):
@@ -137,7 +151,7 @@ class PowerSpherical(Distribution):
 
     def log_normalizer(self):
         # log C(kappa) = -((a+b) ln 2 + lgamma(a) - lgamma(a+b) + b ln pi) evaluated on the device
-        return ops.PSLogNormalizer.apply(self.scale, self.dim)
+        return ops.ps_log_normalizer(self.scale, self.dim)
 
     def log_prob(self, value):
         loc2, kap = self._flat()
@@ -149,13 +163,9 @@ class PowerSpherical(Distribution):
 
     def entropy(self):
         cached = self._fused_entropy
-        if cached is not None:
-            param = self._raw_scale if self._head is not None else self.scale
-            stale = (torch.is_grad_enabled() and torch.is_tensor(param) and param.requires_grad
-                     and cached.grad_fn is None and not cached.requires_grad)
-            if not stale:
-                return cached.to(self.loc.dtype)
-        ent = ops.PSEntropy.apply(self.scale, 1, (self.dim - 1) / 2, False)
+        if cached is not None and not _stale(cached, self._raw_scale if self._head is not None else self.scale):
+            return cached.to(self.loc.dtype)
+        ent = ops.ps_entropy(self.scale, 1, (self.dim - 1) / 2, False)
         return ent.reshape(self.scale.shape).to(self.loc.dtype)
 
 
@@ -230,10 +240,9 @@ class CliffordTorusDistribution(Distribution):
         n = _numel(sample_shape)
         loc2 = self.loc.reshape(-1, d)
         kap = self._vm_kappa(row_scalar_if_expanded=True)
-        if torch.is_grad_enabled() and (loc2.requires_grad or kap.requires_grad):
+        if ops._wants_graph(loc2, kap):
             z, ent, dent = ops.CliffordVMRsample.apply(loc2, kap, n, True)
-            if ent.numel():                                         # same launch; entropy() / kl_divergence reuse it
-                self._fused_entropy = ops.row_scalar(kap, ent, dent).reshape(self.batch_shape)
+            _keep_fused(self, "_fused_entropy", kap, self.batch_shape, (ent, dent))
         else:
             z = ops.clifford_vm_rsample(loc2, self._vm_kappa(), n)
         return z.reshape(tuple(sample_shape) + tuple(self.batch_shape) + (2 * d,)).to(self.loc.dtype)
@@ -247,15 +256,10 @@ class CliffordTorusDistribution(Distribution):
 
     def entropy(self):
         cached = self.__dict__.get("_fused_entropy")
-        if cached is not None:
-            # a value cached without a graph carries none: recompute when the caller now wants d entropy / d kappa
-            kap = self._vm_kappa(row_scalar_if_expanded=True)
-            stale = torch.is_grad_enabled() and kap.requires_grad and cached.grad_fn is None and not cached.requires_grad
-            if not stale:
-                return cached.to(self.loc.dtype)
+        if cached is not None and not _stale(cached, self._vm_kappa(row_scalar_if_expanded=True)):
+            return cached.to(self.loc.dtype)
         # one kernel: sum over circles k >= 1 of ln 2 pi + ln(i0e + eps) + kappa - kappa (i1e + eps) / (i0e + eps)
-        d = self.orig_dim
-        ent = ops.VMTorusEntropy.apply(self._vm_kappa(), d)
+        ent = ops.vm_torus_entropy(self._vm_kappa(), self.orig_dim)
         return ent.reshape(self.batch_shape).to(self.loc.dtype)
 
 
@@ -334,17 +338,15 @@ class CliffordPowerSphericalDistribution(CliffordTorusDistribution):
         out_shape = tuple(sample_shape) + tuple(self.batch_shape) + (2 * d,)
         if _base_draws is None:
             _base_draws = testing.take()
-        if self._head is not None and torch.is_grad_enabled() and (self.loc.requires_grad or self._raw_scale.requires_grad):
+        if self._head is not None and ops._wants_graph(self.loc, self._raw_scale):
             # training path from the raw head output: softplus + floor + clamp inside the kernel
             raw2 = self._raw_scale.reshape(-1, 1)
             z, ent, dent = ops.CliffordPSRsample.apply(self.loc.reshape(-1, d), raw2, n, _base_draws, True, self._head)
-            if ent.numel():
-                self._fused_entropy = ops.row_scalar(raw2, ent, dent).reshape(self.batch_shape)
+            _keep_fused(self, "_fused_entropy", raw2, self.batch_shape, (ent, dent))
             return z.reshape(out_shape).to(self.dtype)
         loc2, kap2 = self._flat()
-        no_grad = not (torch.is_grad_enabled() and (loc2.requires_grad or kap2.requires_grad))
-        if (no_grad and len(sample_shape) > 0 and kap2.shape[-1] == 1 and 16 <= d <= 8192 and (d & (d - 1)) == 0
-                and loc2.shape[0] > 0 and n > 0):
+        if (not ops._wants_graph(loc2, kap2) and len(sample_shape) > 0 and kap2.shape[-1] == 1 and 16 <= d <= 8192
+                and (d & (d - 1)) == 0 and loc2.shape[0] > 0 and n > 0):
             # evaluation path (IWAE, mnist/mlp_vae.py:161,181: q_z.rsample(torch.Size([n_samples])) then
             # q_z.log_prob(z)): the same launch also yields log q(z) of the sample, which log_prob() returns when it
             # is handed this very tensor back.  A plain rsample() (empty sample_shape) skips it.
@@ -355,8 +357,7 @@ class CliffordPowerSphericalDistribution(CliffordTorusDistribution):
             self._sample_log_prob = (weakref.ref(z), z._version, lp.reshape(out_shape[:-1]))
             return z
         z, ent, dent = ops.CliffordPSRsample.apply(loc2, kap2, n, _base_draws, True)
-        if ent.numel():
-            self._fused_entropy = ops.row_scalar(kap2, ent, dent).reshape(self.batch_shape)
+        _keep_fused(self, "_fused_entropy", kap2, self.batch_shape, (ent, dent))
         return z.reshape(out_shape).to(self.dtype)
 
     def rsample_bind(self, other, sample_shape=torch.Size(), return_sample=True, _base_draws=None):
@@ -380,15 +381,15 @@ class CliffordPowerSphericalDistribution(CliffordTorusDistribution):
         oth = other if other.numel() == 2 * d else other.expand(out_shape)
         with torch.no_grad():
             z, bound, ent = ops.clifford_rsample_bind(loc2, kap2, oth, n, _base_draws, return_sample)
-        if ent is not None and not (kap2.requires_grad and torch.is_grad_enabled()):
+        if ent is not None and not ops._wants_graph(kap2):
             self._fused_entropy = ent.reshape(self.batch_shape)     # forward-only value: never cached under autograd
         bound = bound.reshape(out_shape).to(self.dtype)
         return (z.reshape(out_shape).to(self.dtype), bound) if return_sample else bound
 
     def log_prob(self, value):
         cached = self._sample_log_prob
-        if cached is not None and cached[0]() is value and value._version == cached[1] and not (
-                torch.is_grad_enabled() and (value.requires_grad or self.loc.requires_grad or self._kappa.requires_grad)):
+        if (cached is not None and cached[0]() is value and value._version == cached[1]
+                and not ops._wants_graph(value, self.loc, self._kappa)):
             return cached[2].to(self.dtype)
         loc2, kap2 = self._flat()
         n = 2 * self.orig_dim
@@ -399,16 +400,10 @@ class CliffordPowerSphericalDistribution(CliffordTorusDistribution):
 
     def entropy(self):
         cached = self._fused_entropy
-        if cached is not None:
-            # a value cached by a no-grad rsample (evaluation path) carries no graph: recompute when the caller now
-            # wants d entropy / d kappa
-            param = self._raw_scale if self._head is not None else self._kappa
-            stale = (torch.is_grad_enabled() and param.requires_grad and cached.grad_fn is None
-                     and not cached.requires_grad)
-            if not stale:
-                return cached.to(self.dtype)
+        if cached is not None and not _stale(cached, self._raw_scale if self._head is not None else self._kappa):
+            return cached.to(self.dtype)
         _, kap2 = self._flat()
-        ent = ops.PSEntropy.apply(kap2, self.orig_dim, 0.5, True)
+        ent = ops.ps_entropy(kap2, self.orig_dim, 0.5, True)
         return ent.reshape(self.batch_shape).to(self.dtype)
 
 

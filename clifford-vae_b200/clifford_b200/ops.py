@@ -46,13 +46,18 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
 
 
 def _prep(*tensors):
-    """Check that all tensors live on one CUDA device (initialising the library there).  Returns (lib, device)."""
+    """Check that all tensors live on one CUDA device (initialising the library there).  Returns the device."""
     dev = tensors[0].device
     _lib.ensure_device(dev)
     for t in tensors[1:]:
         if t is not None and t.device != dev:
             raise _lib.CliffordB200Error(f"tensors on different devices: {dev} vs {t.device}")
-    return _lib.load(), dev
+    return dev
+
+
+def _wants_graph(*tensors) -> bool:
+    """Autograd is recording and one of `tensors` requires grad."""
+    return torch.is_grad_enabled() and any(t.requires_grad for t in tensors)
 
 
 def _kappa_layout(kappa: torch.Tensor, d: int):
@@ -64,15 +69,63 @@ def _kappa_layout(kappa: torch.Tensor, d: int):
     return k, d, 1
 
 
+def _concentration(head, B, *layout):
+    """(entry-point suffix, concentration arguments) of a sampler launch and its backward: `layout` (the torus's kappa
+    row and element strides, nothing on the sphere) and B for a concentration tensor; B, floor, kmax and the `_head`
+    entry points for the raw output of the concentration layer, head = (floor, kmax)."""
+    if head is None:
+        return "", (*layout, B)
+    return "_head", (B, float(head[0]), float(head[1]))
+
+
+def _draws(dev, draws, *shapes, dtypes=None):
+    """The random input of one sampling launch, as (*tensors, seed, offset).  Injected `draws` (a tensor or a tuple of
+    them; a None entry stays None) are reshaped to `shapes` as contiguous tensors of `dtypes` (fp32 by default), with
+    seed = offset = 0.  Without them every tensor is None and the launch draws on the device from one next_rng()."""
+    if draws is None:
+        return (None,) * len(shapes) + _lib.next_rng(dev)
+    if torch.is_tensor(draws):
+        draws = (draws,)
+    dtypes = dtypes or (torch.float32,) * len(shapes)
+    tensors = tuple(None if t is None else t.reshape(s).to(dt).contiguous() for t, s, dt in zip(draws, shapes, dtypes))
+    return tensors + (0, 0)
+
+
+def _sample_sum(t, B):
+    """t (S * B, ...) summed over the S samples of each of the B loc rows; t itself when S == 1."""
+    if t.shape[0] == B:
+        return t
+    return t.view(t.shape[0] // B, B, *t.shape[1:]).sum(0)
+
+
+def _rsample_backward(ctx, grad_z, loc_c, kap_c, *draw_args, snap=None):
+    """(d loc, d kappa) of a sampler from the gradient of its sample z (rows, 2d | D): the backward entry point
+    ctx.entry with (grad_z, loc, kappa, *ctx.conc, *draw_args, dloc (rows, width), dkappa (rows,) | (rows, d)), summed
+    over the samples of each loc row, dkappa shaped like the concentration (ctx.kshape).  The launch runs under
+    replay_counter(snap): in CUDA-graph capture the sphere samplers' backward regenerates the forward's normals from the
+    launch counter snapshot."""
+    if grad_z is None:
+        return (torch.zeros_like(loc_c) if ctx.needs_input_grad[0] else None), None
+    gz = _f32c(grad_z)
+    (rows, _), (B, w) = gz.shape, loc_c.shape
+    dloc = torch.empty(rows, w, device=gz.device, dtype=torch.float32)
+    dk = torch.empty(rows, *kap_c.shape[1:], device=gz.device, dtype=torch.float32)
+    with _lib.replay_counter(gz.device, snap):
+        _launch(ctx.entry, gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), *ctx.conc, *draw_args, ptr(dloc), ptr(dk),
+                rows, w, skip=gz.numel() == 0)
+    return _sample_sum(dloc, B), _sample_sum(dk, B).reshape(ctx.kshape)
+
+
 class RowScalarOfKappa(torch.autograd.Function):
-    """A per-row scalar (entropy, log-normaliser) that a sampler launch already produced, re-attached to the graph as a
-    function of the concentration: forward hands back the precomputed value, backward multiplies by the derivative the
-    same launch produced.  Its own autograd node (own saved tensors), so the sample and the entropy / KL can be
-    differentiated in separate backward passes, like the reference's independent graphs."""
+    """A per-row scalar (entropy, log-normaliser) that a launch already produced, re-attached to the graph as a function
+    of the concentration: forward hands back the precomputed value, backward multiplies by the derivative the same
+    launch produced -- one per value, or (B, d) for a row value of a per-element kappa (B, d).  Its own autograd node
+    (own saved tensors), so the sample and the entropy / KL can be differentiated in separate backward passes, like the
+    reference's independent graphs."""
 
     @staticmethod
     def forward(ctx, kappa, box):
-        value, dvalue = box              # plain tensors made inside the sampler's forward (not inputs of this node)
+        value, dvalue = box              # plain tensors made by the launch (not inputs of this node)
         ctx.save_for_backward(dvalue)
         ctx.kshape = tuple(kappa.shape)
         return value
@@ -80,12 +133,15 @@ class RowScalarOfKappa(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad):
         (dvalue,) = ctx.saved_tensors
-        return (grad.reshape(-1) * dvalue.reshape(-1)).reshape(ctx.kshape), None
+        g = grad.reshape(-1)
+        if dvalue.dim() == 2:
+            g = g[:, None]
+        return (g * dvalue).reshape(ctx.kshape), None
 
 
 def row_scalar(kappa, value, dvalue):
     """value as a differentiable function of kappa when that is wanted, else the bare value."""
-    if torch.is_grad_enabled() and torch.is_tensor(kappa) and kappa.requires_grad:
+    if _wants_graph(kappa):
         return RowScalarOfKappa.apply(kappa, (value, dvalue))
     return value
 
@@ -107,35 +163,25 @@ class CliffordPSRsample(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, loc, kappa, n_samples, draws, want_entropy, head=None):
-        lib, dev = _prep(loc, kappa)
+        dev = _prep(loc, kappa)
         B, d = loc.shape
         rows = B * n_samples
         loc_c = _f32c(loc)
         kap_c, krs, kes = _kappa_layout(kappa, d)
         if head is not None and kes != 0:
             raise NotImplementedError("the folded concentration head needs one raw value per row, shape (B, 1)")
+        sfx, conc = _concentration(head, B, krs, kes)
         z = torch.empty(rows, 2 * d, device=dev, dtype=torch.float32)
         need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         fused_ent = bool(want_entropy) and kes == 0 and n_samples == 1
         ent = torch.empty(B, device=dev, dtype=torch.float32) if fused_ent else None
         dent = torch.empty(B, device=dev, dtype=torch.float32) if fused_ent else None
-        if draws is None:
-            tp = g = None
-            tp_signed = torch.empty(rows, d, device=dev, dtype=torch.float32) if need_grad else None
-            seed, off = _lib.next_rng(dev)
-        else:
-            tp, g = (_f32c(t.reshape(rows, d)) for t in draws)
-            tp_signed = None
-            seed, off = 0, 0
-        if head is None:
-            _launch("cvb_clifford_ps_rsample", dev, ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(tp), ptr(g), seed, off, ptr(z),
-                    ptr(tp_signed), ptr(ent), None, ptr(dent), rows, d, skip=rows == 0 or d == 0)
-        else:
-            _launch("cvb_clifford_ps_rsample_head", dev, ptr(loc_c), ptr(kap_c), B, float(head[0]), float(head[1]), ptr(tp),
-                    ptr(g), seed, off, ptr(z), ptr(tp_signed), ptr(ent), None, ptr(dent), rows, d, skip=rows == 0 or d == 0)
+        tp_signed = torch.empty(rows, d, device=dev, dtype=torch.float32) if draws is None and need_grad else None
+        tp, g, seed, off = _draws(dev, draws, (rows, d), (rows, d))
+        _launch("cvb_clifford_ps_rsample" + sfx, dev, ptr(loc_c), ptr(kap_c), *conc, ptr(tp), ptr(g), seed, off, ptr(z),
+                ptr(tp_signed), ptr(ent), None, ptr(dent), rows, d, skip=rows == 0 or d == 0)
         ctx.save_for_backward(loc_c, kap_c, tp, g, tp_signed)
-        ctx.head = head
-        ctx.meta = (B, d, rows, n_samples, krs, kes, tuple(kappa.shape))
+        ctx.entry, ctx.conc, ctx.kshape = "cvb_clifford_ps_rsample_backward" + sfx, conc, tuple(kappa.shape)
         if ent is None:
             ent, dent = z.new_empty(0), z.new_empty(0)
         ctx.mark_non_differentiable(ent, dent)      # re-attached to kappa by row_scalar(): its own autograd node
@@ -144,31 +190,15 @@ class CliffordPSRsample(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_z, grad_ent, grad_dent):
         loc_c, kap_c, tp, g, tp_signed = ctx.saved_tensors
-        B, d, rows, n_samples, krs, kes, kshape = ctx.meta
-        dloc = dkap = None
         if grad_z is not None:
-            gz = _f32c(grad_z)
-            if gz.data_ptr() % 16:
+            grad_z = _f32c(grad_z)
+            if grad_z.data_ptr() % 16:
                 # a contiguous view at an odd offset (e.g. the gradient of torch.cat([s.view(1), z.flatten()])): the FFT
                 # engine needs 8-byte aligned gradient rows, and at power-of-two d >= 512 the saved device draws can only
-                # be read there (the library refuses the call otherwise)
-                gz = gz.clone()
-            dloc_rows = torch.empty(rows, d, device=gz.device, dtype=torch.float32)
-            dk_rows = torch.empty((rows,) if kes == 0 else (rows, d), device=gz.device, dtype=torch.float32)
-            if ctx.head is None:
-                _launch("cvb_clifford_ps_rsample_backward", gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(tp),
-                        ptr(g), ptr(tp_signed), ptr(dloc_rows), ptr(dk_rows), rows, d, skip=rows == 0 or d == 0)
-            else:
-                _launch("cvb_clifford_ps_rsample_backward_head", gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), B,
-                        float(ctx.head[0]), float(ctx.head[1]), ptr(tp), ptr(g), ptr(tp_signed), ptr(dloc_rows),
-                        ptr(dk_rows), rows, d, skip=rows == 0 or d == 0)
-            if n_samples > 1:
-                dloc_rows = dloc_rows.view(n_samples, B, d).sum(0)
-                dk_rows = dk_rows.view(n_samples, B, -1).sum(0) if kes else dk_rows.view(n_samples, B).sum(0)
-            dloc = dloc_rows
-            dkap = dk_rows.reshape(kshape)
-        if dloc is None and ctx.needs_input_grad[0]:
-            dloc = torch.zeros_like(loc_c)
+                # be read there (the library refuses the call otherwise).  The von Mises backward reads its saved
+                # offsets the same way on every kernel tier and needs no such copy.
+                grad_z = grad_z.clone()
+        dloc, dkap = _rsample_backward(ctx, grad_z, loc_c, kap_c, ptr(tp), ptr(g), ptr(tp_signed))
         return dloc, dkap, None, None, None, None
 
 
@@ -176,7 +206,7 @@ def clifford_rsample_bind(loc, kappa, other, n_samples=1, draws=None, want_sampl
     """Fused forward-only op: z ~ CliffordPS(loc (B,d), kappa (B,1)) for n_samples * B rows, bound = bind(z, other)
     with other (1 | rows, 2d).  Returns (z | None, bound, entropy (B,) | None).  No autograd (evaluation / VSA
     workloads on fresh latents); raises NotImplementedError for shapes the fused kernel does not cover."""
-    lib, dev = _prep(loc, kappa, other)
+    dev = _prep(loc, kappa, other)
     B, d = loc.shape
     rows = B * n_samples
     if kappa.shape[-1] != 1:
@@ -187,12 +217,7 @@ def clifford_rsample_bind(loc, kappa, other, n_samples=1, draws=None, want_sampl
     z = torch.empty(rows, 2 * d, device=dev, dtype=torch.float32) if want_sample else None
     bound = torch.empty(rows, 2 * d, device=dev, dtype=torch.float32)
     ent = torch.empty(B, device=dev, dtype=torch.float32) if n_samples == 1 else None
-    if draws is None:
-        tp = g = None
-        seed, off = _lib.next_rng(dev)
-    else:
-        tp, g = (_f32c(t.reshape(rows, d)) for t in draws)
-        seed, off = 0, 0
+    tp, g, seed, off = _draws(dev, draws, (rows, d), (rows, d))
     _launch("cvb_clifford_ps_rsample_bind", dev, ptr(loc_c), ptr(kap_c), B, ptr(tp), ptr(g), seed, off, ptr(oth_c),
             oth_c.shape[0], ptr(z), ptr(bound), ptr(ent), None, None, rows, d, skip=rows == 0 or d == 0)
     return z, bound, ent
@@ -202,7 +227,7 @@ def clifford_rsample_log_prob(loc, kappa, n_samples=1, draws=None):
     """Fused forward-only op for the IWAE / evaluation path: z ~ CliffordPS(loc (B,d), kappa (B,1)) for n_samples * B
     rows together with log q(z) of every row (the sampler knows its own phases: no FFT -> angle pass over z).
     Returns (z (rows, 2d), log_prob (rows,), entropy (B,) | None).  Power-of-two d in [16, 8192]."""
-    lib, dev = _prep(loc, kappa)
+    dev = _prep(loc, kappa)
     B, d = loc.shape
     rows = B * n_samples
     if kappa.shape[-1] != 1:
@@ -211,51 +236,32 @@ def clifford_rsample_log_prob(loc, kappa, n_samples=1, draws=None):
     z = torch.empty(rows, 2 * d, device=dev, dtype=torch.float32)
     lp = torch.empty(rows, device=dev, dtype=torch.float32)
     ent = torch.empty(B, device=dev, dtype=torch.float32) if n_samples == 1 else None
-    if draws is None:
-        tp = g = None
-        seed, off = _lib.next_rng(dev)
-    else:
-        tp, g = (_f32c(t.reshape(rows, d)) for t in draws)
-        seed, off = 0, 0
+    tp, g, seed, off = _draws(dev, draws, (rows, d), (rows, d))
     _launch("cvb_clifford_ps_rsample_log_prob", dev, ptr(loc_c), ptr(kap_c), B, ptr(tp), ptr(g), seed, off, ptr(z),
             ptr(lp), ptr(ent), None, rows, d, skip=rows == 0 or d == 0)
     return z, lp, ent
 
 
-class PSEntropy(torch.autograd.Function):
-    """Power-spherical entropy per row.  torus=True: sum over circles k>=1 of kappa (B,1)|(B,d)
+def ps_entropy(kappa, d, half_dm1, torus):
+    """Power-spherical entropy per row, differentiable in kappa.  torus=True: sum over circles k>=1 of kappa (B,1)|(B,d)
     (dists/clifford.py:318-322).  torus=False: one D-dim PowerSpherical per row, kappa (B,)."""
-
-    @staticmethod
-    def forward(ctx, kappa, d, half_dm1, torus):
-        lib, dev = _prep(kappa)
-        if torus:
-            kap_c, krs, kes = _kappa_layout(kappa, d)
-            B = kap_c.shape[0]
-        else:
-            kap_c, krs, kes = _f32c(kappa.reshape(-1)), 1, 0
-            B = kap_c.shape[0]
-        ent = torch.empty(B, device=dev, dtype=torch.float32)
-        dent = torch.empty((B,) if kes == 0 else (B, d), device=dev, dtype=torch.float32)
-        _launch("cvb_ps_entropy_kl", dev, ptr(kap_c), krs, kes, B, d, float(half_dm1), 1 if torus else 0, 0.0, ptr(ent),
-                None, ptr(dent), skip=B == 0)
-        ctx.save_for_backward(dent)
-        ctx.kshape = tuple(kappa.shape)
-        ctx.kes = kes
-        return ent
-
-    @staticmethod
-    def backward(ctx, grad):
-        (dent,) = ctx.saved_tensors
-        g = grad.reshape(-1)
-        dk = g * dent if ctx.kes == 0 else g[:, None] * dent
-        return dk.reshape(ctx.kshape), None, None, None
+    dev = _prep(kappa)
+    if torus:
+        kap_c, krs, kes = _kappa_layout(kappa, d)
+    else:
+        kap_c, krs, kes = _f32c(kappa.reshape(-1)), 1, 0
+    B = kap_c.shape[0]
+    ent = torch.empty(B, device=dev, dtype=torch.float32)
+    dent = torch.empty_like(kap_c)
+    _launch("cvb_ps_entropy_kl", dev, ptr(kap_c), krs, kes, B, d, float(half_dm1), 1 if torus else 0, 0.0, ptr(ent),
+            None, ptr(dent), skip=B == 0)
+    return row_scalar(kappa, ent, dent)
 
 
 def _torus_log_prob_forward(ctx, entry, value, loc, kappa):
     """The launch of a Clifford-torus log_prob (`entry`: the power-spherical or the von Mises family) with the derivative
     outputs autograd will need, saved on ctx for _torus_log_prob_backward."""
-    lib, dev = _prep(value, loc, kappa)
+    dev = _prep(value, loc, kappa)
     B, d = loc.shape
     rows = value.shape[0]
     val_c, loc_c = _f32c(value), _f32c(loc)
@@ -275,7 +281,6 @@ def _torus_log_prob_forward(ctx, entry, value, loc, kappa):
 def _torus_log_prob_backward(ctx, grad):
     dl, dk, dF = ctx.saved_tensors
     B, d, rows, kes, kshape = ctx.meta
-    S = rows // B if B else 0
     g = grad.reshape(rows)
     dval = dloc = dkap = None
     if dF is not None:
@@ -283,8 +288,8 @@ def _torus_log_prob_backward(ctx, grad):
         dval = torch.empty(rows, 2 * d, device=g.device, dtype=torch.float32)
         _launch("cvb_clifford_spectrum_adjoint", g.device, ptr(h), ptr(dval), rows, d, skip=rows == 0 or d == 0)
     if dl is not None:
-        dloc = (g[:, None] * dl).view(S, B, d).sum(0)
-        dkap = ((g * dk).view(S, B).sum(0) if kes == 0 else (g[:, None] * dk).view(S, B, d).sum(0)).reshape(kshape)
+        dloc = _sample_sum(g[:, None] * dl, B)
+        dkap = _sample_sum(g * dk if kes == 0 else g[:, None] * dk, B).reshape(kshape)
     return dval, dloc, dkap
 
 
@@ -323,7 +328,7 @@ class CliffordVMRsample(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, loc, kappa, n_samples, want_entropy):
-        lib, dev = _prep(loc, kappa)
+        dev = _prep(loc, kappa)
         B, d = loc.shape
         rows = B * n_samples
         loc_c = _f32c(loc)
@@ -338,7 +343,7 @@ class CliffordVMRsample(torch.autograd.Function):
         _launch("cvb_clifford_vm_rsample_kl", dev, ptr(loc_c), ptr(kap_c), krs, kes, B, seed, off, ptr(z), ptr(phi),
                 ptr(ent), None, ptr(dent), rows, d, skip=rows == 0 or d == 0)
         ctx.save_for_backward(loc_c, kap_c, phi)
-        ctx.meta = (B, d, rows, n_samples, krs, kes, tuple(kappa.shape))
+        ctx.entry, ctx.conc, ctx.kshape = "cvb_clifford_vm_rsample_backward", (krs, kes, B), tuple(kappa.shape)
         if ent is None:
             ent, dent = z.new_empty(0), z.new_empty(0)
         ctx.mark_non_differentiable(ent, dent)      # re-attached to kappa by row_scalar(): its own autograd node
@@ -347,29 +352,14 @@ class CliffordVMRsample(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_z, grad_ent, grad_dent):
         loc_c, kap_c, phi = ctx.saved_tensors
-        B, d, rows, n_samples, krs, kes, kshape = ctx.meta
-        dloc = dkap = None
-        if grad_z is not None and phi is not None:
-            gz = _f32c(grad_z)
-            dloc_rows = torch.empty(rows, d, device=gz.device, dtype=torch.float32)
-            dk_rows = torch.empty((rows,) if kes == 0 else (rows, d), device=gz.device, dtype=torch.float32)
-            _launch("cvb_clifford_vm_rsample_backward", gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), krs, kes, B, ptr(phi),
-                    ptr(dloc_rows), ptr(dk_rows), rows, d, skip=rows == 0 or d == 0)
-            if n_samples > 1:
-                dloc_rows = dloc_rows.view(n_samples, B, d).sum(0)
-                dk_rows = dk_rows.view(n_samples, B, -1).sum(0) if kes else dk_rows.view(n_samples, B).sum(0)
-            dloc = dloc_rows
-            dkap = dk_rows.reshape(kshape)
-        if dloc is None and ctx.needs_input_grad[0]:
-            dloc = torch.zeros_like(loc_c)
-        return dloc, dkap, None, None
+        return (*_rsample_backward(ctx, grad_z, loc_c, kap_c, ptr(phi)), None, None)
 
 
 def clifford_vm_rsample(loc, kappa, n_samples=1):
     """z (n_samples * B, 2d) of the von Mises torus distribution (dists/clifford.py:261-275): phases loc + VonMises(0, kappa)
     drawn on the device, then the Hermitian-spectrum inverse FFT.  loc (B, d), kappa (B, 1) | (B, d).  Forward only (the
     sampling path without a graph); CliffordVMRsample draws the same z with a backward."""
-    lib, dev = _prep(loc, kappa)
+    dev = _prep(loc, kappa)
     B, d = loc.shape
     rows = B * n_samples
     loc_c = _f32c(loc.detach())
@@ -386,11 +376,7 @@ def clifford_phases_to_vector(phases, scale, rows, d, device):
     _lib.ensure_device(torch.device(device))
     z = torch.empty(rows, 2 * d, device=device, dtype=torch.float32)
     dev = z.device
-    if phases is None:
-        seed, off = _lib.next_rng(dev)
-        ph = None
-    else:
-        ph, seed, off = _f32c(phases.reshape(rows, d)), 0, 0
+    ph, seed, off = _draws(dev, phases, (rows, d))
     _launch("cvb_clifford_phases_to_vector", dev, ptr(ph), float(scale), seed, off, ptr(z), rows, d,
             skip=rows == 0 or d == 0)
     return z
@@ -480,7 +466,7 @@ class Bind(torch.autograd.Function):
 
 
 def invert(a):
-    lib, dev = _prep(a)
+    dev = _prep(a)
     d = a.shape[-1]
     a2 = _f32c(a).reshape(-1, d)
     out = torch.empty_like(a2)
@@ -499,7 +485,7 @@ class Invert(torch.autograd.Function):
 
 
 def permute(v, perm, inverse):
-    lib, dev = _prep(v, perm)
+    dev = _prep(v, perm)
     d = v.shape[-1]
     if perm.numel() != d:
         raise ValueError("permutation length must equal the vector dimension")
@@ -526,13 +512,14 @@ class Permute(torch.autograd.Function):
 class Bundle(torch.autograd.Function):
     @staticmethod
     def forward(ctx, vectors, scale):
-        lib, dev = _prep(vectors)
+        dev = _prep(vectors)
         k = vectors.shape[0]
         inner = tuple(vectors.shape[1:])
         d = int(math.prod(inner)) if inner else 1
         v2 = _f32c(vectors).reshape(k, d)
         out = torch.empty(d, device=dev, dtype=torch.float32)
-        ws = torch.empty(max(int(lib.cvb_vsa_bundle_workspace_bytes(k, d)) // 4, 1), device=dev, dtype=torch.float32)
+        ws_bytes = int(_lib.load().cvb_vsa_bundle_workspace_bytes(k, d))
+        ws = torch.empty(max(ws_bytes // 4, 1), device=dev, dtype=torch.float32)
         if k == 0:
             out.zero_()           # an empty stack sums to zero (torch.sum over an empty dim)
         _launch("cvb_vsa_bundle", dev, ptr(v2), ptr(out), k, d, float(scale), ptr(ws), skip=_any_empty(v2))
@@ -548,7 +535,7 @@ class Bundle(torch.autograd.Function):
 class Cosine(torch.autograd.Function):
     @staticmethod
     def forward(ctx, a, b):
-        lib, dev = _prep(a, b)
+        dev = _prep(a, b)
         a2, b2, rows, out_shape = _flatten_pair(a, b)
         d = out_shape[-1]
         out = torch.empty(rows, device=dev, dtype=torch.float32)
@@ -580,7 +567,7 @@ class Cosine(torch.autograd.Function):
 class Normalize(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x):
-        lib, dev = _prep(x)
+        dev = _prep(x)
         d = x.shape[-1]
         x2 = _f32c(x).reshape(-1, d)
         out = torch.empty_like(x2)
@@ -627,11 +614,7 @@ def sphere_uniform_rsample(rows, D, device, norm_eps, gnoise=None):
     _lib.ensure_device(dev)
     z = torch.empty(rows, D, device=dev, dtype=torch.float32)
     dev = z.device
-    if gnoise is None:
-        seed, off = _lib.next_rng(dev)
-        g = None
-    else:
-        g, seed, off = _f32c(gnoise.reshape(rows, D)), 0, 0
+    g, seed, off = _draws(dev, gnoise, (rows, D))
     _launch("cvb_sphere_uniform_rsample", dev, ptr(g), seed, off, ptr(z), rows, D, float(norm_eps), skip=z.numel() == 0)
     return z
 
@@ -639,64 +622,43 @@ def sphere_uniform_rsample(rows, D, device, norm_eps, gnoise=None):
 class PowerSphericalRsample(torch.autograd.Function):
     """(z (n*B, D), entropy (B,), d entropy / d kappa (B,)) = PowerSpherical(loc (B,D), kappa (B,)).rsample fused with
     .entropy() in ONE launch (the training step evaluates both, mnist/mlp_vae.py:110-129); the two row scalars are plain
-    values re-attached to kappa by row_scalar().  draws None or (tprime (rows,), g (rows, D-1))."""
+    values re-attached to kappa by row_scalar().  draws None or (tprime (rows,), g (rows, D-1)).
+    head = (floor, kmax): `kappa` is the raw layer output, as in CliffordPSRsample."""
 
     @staticmethod
     def forward(ctx, loc, kappa, n_samples, draws, head=None):
-        lib, dev = _prep(loc, kappa)
+        dev = _prep(loc, kappa)
         B, D = loc.shape
         rows = B * n_samples
         loc_c, kap_c = _f32c(loc), _f32c(kappa.reshape(-1))
+        sfx, conc = _concentration(head, B)
         z = torch.empty(rows, D, device=dev, dtype=torch.float32)
         ent = torch.empty(B, device=dev, dtype=torch.float32)
         dent = torch.empty(B, device=dev, dtype=torch.float32)
-        hd = () if head is None else (float(head[0]), float(head[1]))      # head: kappa is the raw layer output
-        sfx = "" if head is None else "_head"
-        snap = None
-        if draws is None:
-            tp = g = None
-            save = torch.empty(rows, 2, device=dev, dtype=torch.float32)
-            seed, off = _lib.next_rng(dev)
-            if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
-                snap = _lib.graph_counter_snapshot(dev)     # the backward replays this launch's normals
-        else:
-            tp = _f32c(draws[0].reshape(rows))
-            g = _f32c(draws[1].reshape(rows, D - 1))
-            save, seed, off = None, 0, 0
-        _launch("cvb_powerspherical_rsample_kl" + sfx, dev, ptr(loc_c), ptr(kap_c), B, *hd, ptr(tp), ptr(g), seed, off, ptr(z),
-                ptr(save), ptr(ent), None, ptr(dent), rows, D, skip=z.numel() == 0)
+        save = torch.empty(rows, 2, device=dev, dtype=torch.float32) if draws is None else None
+        tp, g, seed, off = _draws(dev, draws, (rows,), (rows, D - 1))
+        need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        # the backward replays this launch's normals
+        ctx.snap = _lib.graph_counter_snapshot(dev) if draws is None and need_grad else None
+        _launch("cvb_powerspherical_rsample_kl" + sfx, dev, ptr(loc_c), ptr(kap_c), *conc, ptr(tp), ptr(g), seed, off,
+                ptr(z), ptr(save), ptr(ent), None, ptr(dent), rows, D, skip=z.numel() == 0)
         ctx.save_for_backward(loc_c, kap_c, tp, g, save)
-        ctx.head = (sfx, hd)
-        ctx.snap = snap
-        ctx.meta = (B, D, rows, n_samples, seed, off, tuple(kappa.shape))
+        ctx.entry, ctx.conc, ctx.kshape = "cvb_powerspherical_rsample_backward" + sfx, conc, tuple(kappa.shape)
+        ctx.rng = (seed, off)
         ctx.mark_non_differentiable(ent, dent)
         return z, ent, dent
 
     @staticmethod
     def backward(ctx, grad_z, grad_ent, grad_dent):
         loc_c, kap_c, tp, g, save = ctx.saved_tensors
-        B, D, rows, n_samples, seed, off, kshape = ctx.meta
-        dloc = dk = None
-        if grad_z is not None:
-            gz = _f32c(grad_z).reshape(rows, D)
-            dloc = torch.empty(rows, D, device=gz.device, dtype=torch.float32)
-            dk = torch.empty(rows, device=gz.device, dtype=torch.float32)
-            sfx, hd = ctx.head
-            with _lib.replay_counter(gz.device, ctx.snap):
-                _launch("cvb_powerspherical_rsample_backward" + sfx, gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), B, *hd, ptr(tp),
-                        ptr(g), ptr(save), seed, off, ptr(dloc), ptr(dk), rows, D, skip=gz.numel() == 0)
-            if n_samples > 1:
-                dloc = dloc.view(n_samples, B, D).sum(0)
-                dk = dk.view(n_samples, B).sum(0)
-        if dloc is None and ctx.needs_input_grad[0]:
-            dloc = torch.zeros_like(loc_c)
-        return dloc, (None if dk is None else dk.reshape(kshape)), None, None, None
+        dloc, dkap = _rsample_backward(ctx, grad_z, loc_c, kap_c, ptr(tp), ptr(g), ptr(save), *ctx.rng, snap=ctx.snap)
+        return dloc, dkap, None, None, None
 
 
 class PowerSphericalLogProb(torch.autograd.Function):
     @staticmethod
     def forward(ctx, value, loc, kappa):
-        lib, dev = _prep(value, loc, kappa)
+        dev = _prep(value, loc, kappa)
         B, D = loc.shape
         rows = value.shape[0]
         val_c, loc_c, kap_c = _f32c(value), _f32c(loc), _f32c(kappa.reshape(-1))
@@ -707,17 +669,15 @@ class PowerSphericalLogProb(torch.autograd.Function):
         _launch("cvb_powerspherical_log_prob", dev, ptr(val_c), ptr(loc_c), ptr(kap_c), B, ptr(lp), ptr(coef), ptr(dk),
                 rows, D, skip=val_c.numel() == 0)
         ctx.save_for_backward(val_c, loc_c, coef, dk)
-        ctx.meta = (B, D, rows, tuple(kappa.shape))
+        ctx.kshape = tuple(kappa.shape)
         return lp
 
     @staticmethod
     def backward(ctx, grad):
         val_c, loc_c, coef, dk = ctx.saved_tensors
-        B, D, rows, kshape = ctx.meta
-        S = rows // B
-        g = _f32c(grad).reshape(rows)
+        g = _f32c(grad).reshape(-1)
         dval, dloc = _logprob_backward(g * coef, val_c, loc_c, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
-        dkap = (g * dk).view(S, B).sum(0).reshape(kshape) if ctx.needs_input_grad[2] else None
+        dkap = _sample_sum(g * dk, loc_c.shape[0]).reshape(ctx.kshape) if ctx.needs_input_grad[2] else None
         return dval, dloc, dkap
 
 
@@ -742,7 +702,7 @@ class VMFLogProb(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, value, loc, kappa, log_norm):
-        lib, dev = _prep(value, loc, kappa, log_norm)
+        dev = _prep(value, loc, kappa, log_norm)
         B, D = loc.shape
         rows = value.shape[0]
         val_c, loc_c, kap_c, ln_c = _f32c(value), _f32c(loc), _f32c(kappa.reshape(-1)), _f32c(log_norm.reshape(-1))
@@ -751,146 +711,91 @@ class VMFLogProb(torch.autograd.Function):
         _launch("cvb_vmf_log_prob", dev, ptr(val_c), ptr(loc_c), ptr(kap_c), ptr(ln_c), B, ptr(lp), ptr(dot), rows, D,
                 skip=val_c.numel() == 0)
         ctx.save_for_backward(val_c, loc_c, kap_c, dot)
-        ctx.meta = (B, D, rows, tuple(kappa.shape), tuple(log_norm.shape))
+        ctx.meta = (tuple(kappa.shape), tuple(log_norm.shape))
         return lp
 
     @staticmethod
     def backward(ctx, grad):
         val_c, loc_c, kap_c, dot = ctx.saved_tensors
-        B, D, rows, kshape, lshape = ctx.meta
-        S = rows // B
-        g = _f32c(grad).reshape(rows)
-        w = (g.view(S, B) * kap_c).reshape(rows)
+        kshape, lshape = ctx.meta
+        B = loc_c.shape[0]
+        g = _f32c(grad).reshape(-1)
+        w = (g.view(-1, B) * kap_c).reshape(-1)
         dval, dloc = _logprob_backward(w, val_c, loc_c, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
-        dkap = (g * dot).view(S, B).sum(0).reshape(kshape) if ctx.needs_input_grad[2] else None
-        dln = (-g.view(S, B).sum(0)).reshape(lshape) if ctx.needs_input_grad[3] else None
+        dkap = _sample_sum(g * dot, B).reshape(kshape) if ctx.needs_input_grad[2] else None
+        dln = (-_sample_sum(g, B)).reshape(lshape) if ctx.needs_input_grad[3] else None
         return dval, dloc, dkap, dln
 
 
-class VMTorusEntropy(torch.autograd.Function):
+def vm_torus_entropy(kappa, d):
     """CliffordTorusDistribution.entropy (dists/clifford.py:21-31, :277-278) per row of kappa (B,1)|(B,d): the sum over
-    circles k >= 1 of the (eps-regularised) von Mises entropy, with its kappa-derivative for the backward."""
-
-    @staticmethod
-    def forward(ctx, kappa, d):
-        lib, dev = _prep(kappa)
-        kap_c, krs, kes = _kappa_layout(kappa, d)
-        B = kap_c.shape[0]
-        ent = torch.empty(B, device=dev, dtype=torch.float32)
-        dent = torch.empty((B,) if kes == 0 else (B, d), device=dev, dtype=torch.float32) if ctx.needs_input_grad[0] else None
-        _launch("cvb_clifford_vm_entropy", dev, ptr(kap_c), krs, kes, B, d, ptr(ent), ptr(dent), skip=B == 0)
-        ctx.save_for_backward(dent)
-        ctx.kshape = tuple(kappa.shape)
-        ctx.kes = kes
-        return ent
-
-    @staticmethod
-    def backward(ctx, grad):
-        (dent,) = ctx.saved_tensors
-        g = grad.reshape(-1)
-        dk = g * dent if ctx.kes == 0 else g[:, None] * dent
-        return dk.reshape(ctx.kshape), None
+    circles k >= 1 of the (eps-regularised) von Mises entropy, differentiable in kappa."""
+    dev = _prep(kappa)
+    kap_c, krs, kes = _kappa_layout(kappa, d)
+    B = kap_c.shape[0]
+    ent = torch.empty(B, device=dev, dtype=torch.float32)
+    dent = torch.empty_like(kap_c) if _wants_graph(kappa) else None
+    _launch("cvb_clifford_vm_entropy", dev, ptr(kap_c), krs, kes, B, d, ptr(ent), ptr(dent), skip=B == 0)
+    return row_scalar(kappa, ent, dent)
 
 
-class PSLogNormalizer(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, kappa, dim):
-        lib, dev = _prep(kappa)
-        k = _f32c(kappa.reshape(-1))
-        ln = torch.empty_like(k)
-        dln = torch.empty_like(k)
-        _launch("cvb_ps_log_normalizer", dev, ptr(k), k.numel(), (dim - 1) / 2, ptr(ln), ptr(dln), skip=k.numel() == 0)
-        ctx.save_for_backward(dln)
-        ctx.kshape = tuple(kappa.shape)
-        return ln.reshape(kappa.shape)
-
-    @staticmethod
-    def backward(ctx, grad):
-        (dln,) = ctx.saved_tensors
-        return (grad.reshape(-1) * dln).reshape(ctx.kshape), None
+def ps_log_normalizer(kappa, dim):
+    """PowerSpherical log-normaliser, elementwise in kappa and differentiable in it."""
+    dev = _prep(kappa)
+    k = _f32c(kappa.reshape(-1))
+    ln = torch.empty(kappa.shape, device=dev, dtype=torch.float32)
+    dln = torch.empty_like(k)
+    _launch("cvb_ps_log_normalizer", dev, ptr(k), k.numel(), (dim - 1) / 2, ptr(ln), ptr(dln), skip=k.numel() == 0)
+    return row_scalar(kappa, ln, dln)
 
 
 class VMFRsample(torch.autograd.Function):
     """(z (rows, D), entropy, log_norm, d entropy / d kappa, d log_norm / d kappa (B,) each) = VonMisesFisher(loc (B,D),
     kappa (B,1)).rsample fused with the row's entropy and log-normaliser (von_mises_fisher.py:183-212) in ONE launch; the
     row scalars are plain values re-attached to kappa by row_scalar().
-    draws: None or (e_rounds (R, rows) f64 | None for D == 3, u_rounds (R, rows) f64, g (rows, D))."""
+    draws: None or (e_rounds (R, rows) f64 | None for D == 3, u_rounds (R, rows) f64, g (rows, D)).
+    head = (floor, kmax): `kappa` is the raw layer output, as in CliffordPSRsample."""
 
     @staticmethod
     def forward(ctx, loc, kappa, n_samples, draws, head=None):
-        lib, dev = _prep(loc, kappa)
+        dev = _prep(loc, kappa)
         B, D = loc.shape
         rows = B * n_samples
         loc_c, kap_c = _f32c(loc), _f32c(kappa.reshape(-1))
-        hd = () if head is None else (float(head[0]), float(head[1]))      # head: kappa is the raw layer output
-        sfx = "" if head is None else "_head"
+        sfx, conc = _concentration(head, B)
         z = torch.empty(rows, D, device=dev, dtype=torch.float32)
         save = torch.empty(rows, 2, device=dev, dtype=torch.float32)
         ent, ln, dent, dln = (torch.empty(B, device=dev, dtype=torch.float32) for _ in range(4))
-        snap = None
-        if draws is None:
-            e = u = g = None
-            R = 0
-            seed, off = _lib.next_rng(dev)
-            if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
-                snap = _lib.graph_counter_snapshot(dev)     # the backward replays this launch's normals
-        else:
-            e, u, g = draws
-            u = u.to(torch.float64).reshape(-1, rows).contiguous()
-            e = None if e is None else e.to(torch.float64).reshape(-1, rows).contiguous()
-            R = u.shape[0]
-            g = _f32c(g.reshape(rows, D))
-            seed, off = 0, 0
-        _launch("cvb_vmf_rsample_kl" + sfx, dev, ptr(loc_c), ptr(kap_c), B, *hd, ptr(e), ptr(u), R, ptr(g), seed, off, ptr(z),
+        e, u, g, seed, off = _draws(dev, draws, (-1, rows), (-1, rows), (rows, D),
+                                    dtypes=(torch.float64, torch.float64, torch.float32))
+        need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        # the backward replays this launch's normals
+        ctx.snap = _lib.graph_counter_snapshot(dev) if draws is None and need_grad else None
+        R = 0 if u is None else u.shape[0]
+        _launch("cvb_vmf_rsample_kl" + sfx, dev, ptr(loc_c), ptr(kap_c), *conc, ptr(e), ptr(u), R, ptr(g), seed, off, ptr(z),
                 ptr(save), ptr(ent), None, ptr(dent), ptr(ln), ptr(dln), rows, D, skip=z.numel() == 0)
         ctx.save_for_backward(loc_c, kap_c, g, save)
-        ctx.head = (sfx, hd)
-        ctx.snap = snap
-        ctx.meta = (B, D, rows, n_samples, seed, off, tuple(kappa.shape))
+        ctx.entry, ctx.conc, ctx.kshape = "cvb_vmf_rsample_backward" + sfx, conc, tuple(kappa.shape)
+        ctx.rng = (seed, off)
         ctx.mark_non_differentiable(ent, ln, dent, dln)
         return z, ent, ln, dent, dln
 
     @staticmethod
     def backward(ctx, grad_z, *unused):
         loc_c, kap_c, g, save = ctx.saved_tensors
-        B, D, rows, n_samples, seed, off, kshape = ctx.meta
-        dloc = dk = None
-        if grad_z is not None:
-            gz = _f32c(grad_z).reshape(rows, D)
-            dloc = torch.empty(rows, D, device=gz.device, dtype=torch.float32)
-            dk = torch.empty(rows, device=gz.device, dtype=torch.float32)
-            sfx, hd = ctx.head
-            with _lib.replay_counter(gz.device, ctx.snap):
-                _launch("cvb_vmf_rsample_backward" + sfx, gz.device, ptr(gz), ptr(loc_c), ptr(kap_c), B, *hd, ptr(g), ptr(save),
-                        seed, off, ptr(dloc), ptr(dk), rows, D, skip=gz.numel() == 0)
-            if n_samples > 1:
-                dloc = dloc.view(n_samples, B, D).sum(0)
-                dk = dk.view(n_samples, B).sum(0)
-        if dloc is None and ctx.needs_input_grad[0]:
-            dloc = torch.zeros_like(loc_c)
-        return dloc, (None if dk is None else dk.reshape(kshape)), None, None, None
+        dloc, dkap = _rsample_backward(ctx, grad_z, loc_c, kap_c, ptr(g), ptr(save), *ctx.rng, snap=ctx.snap)
+        return dloc, dkap, None, None, None
 
 
-class VMFEntropyLogNorm(torch.autograd.Function):
-    """(entropy, log_norm) per row of kappa (B,1) for sphere dimension D."""
+class VMFEntropyLogNorm:
+    """(entropy, log_norm) per row of kappa (B,1) for sphere dimension D from one launch, each its own differentiable
+    function of kappa (row_scalar).  Called as VMFEntropyLogNorm.apply(kappa, D), like an autograd Function."""
 
     @staticmethod
-    def forward(ctx, kappa, D):
-        lib, dev = _prep(kappa)
+    def apply(kappa, D):
+        dev = _prep(kappa)
         k = _f32c(kappa.reshape(-1))
         ent, ln, dent, dln = (torch.empty_like(k) for _ in range(4))
         _launch("cvb_vmf_entropy_lognorm", dev, ptr(k), k.numel(), D, ptr(ent), ptr(ln), ptr(dent), ptr(dln),
                 skip=k.numel() == 0)
-        ctx.save_for_backward(dent, dln)
-        ctx.kshape = tuple(kappa.shape)
-        return ent, ln
-
-    @staticmethod
-    def backward(ctx, g_ent, g_ln):
-        dent, dln = ctx.saved_tensors
-        out = torch.zeros_like(dent)
-        if g_ent is not None:
-            out = out + g_ent.reshape(-1) * dent
-        if g_ln is not None:
-            out = out + g_ln.reshape(-1) * dln
-        return out.reshape(ctx.kshape), None
+        return row_scalar(kappa, ent, dent), row_scalar(kappa, ln, dln)

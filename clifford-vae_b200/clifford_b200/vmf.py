@@ -11,6 +11,7 @@ import torch
 from torch.distributions.kl import register_kl
 
 from . import ops, testing
+from .distributions import _keep_fused, _stale, head_concentration
 
 
 class HypersphericalUniform(torch.distributions.Distribution):
@@ -100,7 +101,6 @@ class VonMisesFisher(torch.distributions.Distribution):
 
     def __getattr__(self, name):
         if name == "scale" and self.__dict__.get("_head") is not None:
-            from .distributions import head_concentration
             self.__dict__["scale"] = head_concentration(self._raw_scale, *self._head)
             return self.__dict__["scale"]
         raise AttributeError(name)
@@ -131,19 +131,14 @@ class VonMisesFisher(torch.distributions.Distribution):
         if _base_draws is None:
             _base_draws = testing.take()
         z, ent, ln, dent, dln = ops.VMFRsample.apply(loc2, kap, n, _base_draws, self._head)
-        if ent.numel() and tuple(param.shape) == tuple(self.loc.shape[:-1]) + (1,):
-            shp = param.shape[:-1]                          # same launch: entropy() / KL / log_prob reuse the row scalars
-            self._fused = (ops.row_scalar(param, ent, dent).reshape(shp), ops.row_scalar(param, ln, dln).reshape(shp))
+        if tuple(param.shape) == tuple(self.loc.shape[:-1]) + (1,):
+            _keep_fused(self, "_fused", param, param.shape[:-1], (ent, dent), (ln, dln))
         return z.reshape(tuple(shape) + tuple(self.loc.shape)).type(self.dtype)
 
     def _ent_ln(self):
         cached = self._fused
-        if cached is not None:
-            param = self._raw_scale if self._head is not None else self.scale
-            stale = (torch.is_grad_enabled() and param.requires_grad and cached[0].grad_fn is None
-                     and not cached[0].requires_grad)
-            if not stale:
-                return cached
+        if cached is not None and not _stale(cached[0], self._raw_scale if self._head is not None else self.scale):
+            return cached
         ent, ln = ops.VMFEntropyLogNorm.apply(self.scale, self._m)
         shp = self.scale.shape[:-1]
         return ent.reshape(shp), ln.reshape(shp)
