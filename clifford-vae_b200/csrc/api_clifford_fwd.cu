@@ -25,6 +25,7 @@ int launch_fwd_fast(const CliffordFwdParams& p, cudaStream_t st) {
 template <int LOG2N, int MODE>
 int launch_fwd_bind(const CliffordFwdParams& p, cudaStream_t st) {
   using Pl = FftPlan<LOG2N>;
+  static_assert(clifford_fwd_smem_bytes<LOG2N, MODE, true>() <= 227 * 1024, "bind kernel exceeds a CTA's shared memory");
   const cplx* tw = device_twiddles();
   const float2* icdf = device_icdf_table();
   if (!tw || !icdf) return kCudaError;

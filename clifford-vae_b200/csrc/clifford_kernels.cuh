@@ -414,6 +414,10 @@ __device__ __forceinline__ void vm_fwd_row_entropies(const CliffordFwdParams& p,
 typedef unsigned short QueueIndex;   // retry-queue entries are bin indices < N <= 8192
 constexpr int kLpSlots = 16;   // per-warp partial sums of the fused log_prob (groups of up to 512 threads)
 constexpr int clifford_fwd_stages(int mode) { return mode == kPsInjected ? 3 : ((mode == kPsRng || mode == kPhases) ? 1 : 0); }
+// The injected-draw bind at d = 8192 reads its inputs with plain loads: three staged rows (96 KB) beside the bind spectrum
+// (64 KB) would exceed the 227 KB a CTA can have.
+template <int LOG2N, int MODE, bool BIND>
+constexpr int clifford_fwd_staged_rows() { return (BIND && MODE == kPsInjected && LOG2N == 13) ? 0 : clifford_fwd_stages(MODE); }
 // Device-RNG rows with one concentration <= kIcdfKappaMax are sampled through the row's inverse-CDF table
 // (icdf_table.cuh) when the row is long enough to amortise building it (d >= 512: 256 cells by >= 32 threads).
 template <int LOG2N, int MODE>
@@ -421,7 +425,7 @@ constexpr bool clifford_fwd_has_icdf() { return MODE == kPsRng && LOG2N >= 9; }
 template <int LOG2N, int MODE, bool BIND = false>
 constexpr size_t clifford_fwd_smem_bytes() {
   using Pl = FftPlan<LOG2N>;
-  return (sizeof(cplx) * Pl::XCH + sizeof(QueueIndex) * Pl::N + sizeof(float) * Pl::N * clifford_fwd_stages(MODE) +
+  return (sizeof(cplx) * Pl::XCH + sizeof(QueueIndex) * Pl::N + sizeof(float) * Pl::N * clifford_fwd_staged_rows<LOG2N, MODE, BIND>() +
           (BIND ? sizeof(cplx) * Pl::N : 0) + (clifford_fwd_has_icdf<LOG2N, MODE>() ? sizeof(float4) * kFwdIcdfCells : 0)) * Pl::GROUPS +
          (sizeof(uint64_t) + sizeof(int) * 2 + sizeof(float) * kLpSlots) * Pl::GROUPS;
 }
@@ -438,7 +442,7 @@ clifford_fwd_kernel(const CliffordFwdParams p, const cplx* __restrict__ tw, cons
   pdl_wait_and_release();
   using Pl = FftPlan<LOG2N>;
   constexpr int d = Pl::N, T = Pl::T, E = Pl::E, G = Pl::GROUPS;
-  constexpr int NST = clifford_fwd_stages(MODE);
+  constexpr int NST = clifford_fwd_staged_rows<LOG2N, MODE, BIND>();
   constexpr bool ICDF = clifford_fwd_has_icdf<LOG2N, MODE>() && ROWK;
   constexpr uint32_t kRowBytes = d * sizeof(float);
   extern __shared__ __align__(16) unsigned char smem_raw[];

@@ -21,7 +21,7 @@ from conftest import rel_err
 
 DEV = "cuda"
 ROW_TILE = [2, 8, 40, 200]
-FFT = [16, 64, 512, 2048, 8192]
+FFT = [16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192]
 DIRECT = [257, 300, 1000, 4097]
 S = 3                                   # samples per loc row in the broadcast cases: rows = S * loc_rows
 GUARD = 64                              # NaN floats before and after every output

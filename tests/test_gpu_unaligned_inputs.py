@@ -11,7 +11,7 @@ from conftest import rel_err
 pytestmark = pytest.mark.gpu
 
 DEV = "cuda"
-DIMS = [16, 512, 2048]
+DIMS = [16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192]
 ROWS = 4099            # enough rows for the CTAs to loop: dynamic schedule and next-row prefetch
 
 
